@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            (our arm; torchrun for N > 1)
   python bench.py --impl reference --gpus N --steps K --warmup W   (reference CPU arm)
+  python bench.py ... --dump-outputs DIR          (also write the records of the last timed step, DIR/<field>.npy)
 
 Workload (BASELINE.json): configs[1] = 1 M x 250 bp Illumina-like query reads against a 10 M-read synthetic
 metagenome on one B200.  For N > 1 the database grows to N x 10 M reads (configs[2] at N = 8: 80 M reads), sharded
@@ -69,7 +70,14 @@ def parse():
                          "N = 1 allowed); default: configs[1] at N = 1 and N x 10M reads (weak) at N > 1")
     ap.add_argument("--parity-sample", type=int, default=1024,
                     help="query reads checked against the index-free oracle after the timed region (0 = skip)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the records of the last step as DIR/<field>.npy (see dump_records)")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes the GPU arm's records: not with --impl reference")
+    return a
 
 
 def workload(scale, cfg3=False, world=1):
@@ -361,6 +369,25 @@ def H_mod():
     return H
 
 
+DUMP_BYTES_MAX = 60_000_000  # array bytes of one --dump-outputs directory: with the .npy headers under 64 MB
+DUMP_FIELDS = (("accepted", "float32"), ("db_seq", "float64"), ("qpos_end", "float64"), ("db_pos", "float64"),
+               ("length", "float32"), ("identities", "float32"))
+
+
+def dump_records(d, rec, np):
+    """The records a caller of the timed path receives (imsame_gpu_fetch: one per query read), one file per field,
+    plus read.npy with the query read each row belongs to.  Read numbers and positions are float64 (exact below
+    2^53), lengths, identities and the accepted flag float32.  Above DUMP_BYTES_MAX, a fixed seeded sample of reads."""
+    per_read = 8 + sum(np.dtype(t).itemsize for _, t in DUMP_FIELDS)
+    reads = np.arange(len(rec))
+    if len(rec) * per_read > DUMP_BYTES_MAX:
+        reads = np.sort(np.random.default_rng(20261020).choice(len(rec), DUMP_BYTES_MAX // per_read, replace=False))
+    os.makedirs(d, exist_ok=True)
+    np.save(os.path.join(d, "read.npy"), reads.astype(np.float64))
+    for name, t in DUMP_FIELDS:
+        np.save(os.path.join(d, name + ".npy"), rec[name][reads].astype(t))
+
+
 # ------------------------------------------------------------------------------------------
 def sampled_parity(n_sample, rec, db, ds, q, qs, db_total_global, rank, world, nd, L, dist, torch, np):
     """AFTER the timed region, checker only: a seeded random sample of query reads (accepted and unaccepted)
@@ -514,6 +541,8 @@ def run_ours(args):
     ms_total = float(tmax.item())
     clocks = sampler.stop() if rank == 0 else None
     rec = ctx.fetch(keys.data_ptr(), payload.data_ptr())
+    if args.dump_outputs and rank == 0:  # every rank holds the reduced records
+        dump_records(args.dump_outputs, rec, np)
     n_accepted = int(rec["accepted"].sum())
     # self-check of the sharded reduction (N > 1): the band-stepped run with key exchanges must give the
     # same records as independent shard runs followed by one min/max reduction

@@ -196,6 +196,11 @@ long double orc_evalue(int64_t n, uint64_t ylen, uint64_t db_total_len) {
     return (long double)0.333 * t_len * db_total_len * expl(-0.275 * rawscore);
 }
 
+/* default -evalue: 1/powl(10,20) in long double, src/IMSAME.c:44 */
+long double orc_default_evalue(void) {
+    return 1 / powl(10, 20);
+}
+
 /* ------------------------------------------------------------------------- */
 /* NW: src/alignmentFunctions.c:389-489, traceback :493-560, rendering and    */
 /* identity count :230-271. X = database read (rows), Y = query read (cols).  */

@@ -71,6 +71,7 @@ int64_t orc_extend(const orc_seqs *db, const orc_seqs *q, uint64_t pos_db, uint6
 int64_t orc_extend_k(const orc_seqs *db, const orc_seqs *q, uint64_t pos_db, uint64_t pos_q,
                      uint64_t read, uint64_t db_seq, int k);
 long double orc_evalue(int64_t n, uint64_t ylen, uint64_t db_total_len);
+long double orc_default_evalue(void);
 
 /* full NW with back-pointers + traceback + rendering (reference formulation) */
 int orc_nw_traceback(const unsigned char *X, uint64_t xlen, const unsigned char *Y, uint64_t ylen,

@@ -60,6 +60,8 @@ def oracle():
                                    C.c_uint64, C.c_uint64]
         lib.orc_evalue.restype = C.c_longdouble
         lib.orc_evalue.argtypes = [C.c_int64, C.c_uint64, C.c_uint64]
+        lib.orc_default_evalue.restype = C.c_longdouble
+        lib.orc_default_evalue.argtypes = []
         u8p = C.POINTER(C.c_ubyte)
         i32p, u32p = C.POINTER(C.c_int32), C.POINTER(C.c_uint32)
         lib.orc_nw_traceback.argtypes = [u8p, C.c_uint64, u8p, C.c_uint64, C.c_int, C.c_int, i32p, u32p,
@@ -83,7 +85,7 @@ def default_params(n_threads=4, evalue=None, coverage=0.5, identity=0.5, igap=5,
     """Thresholds exactly as src/IMSAME.c:44-47,552-569 derives them."""
     p = OrcParams()
     if evalue is None:
-        p.min_e_value = _ld_default_evalue()
+        p.min_e_value = oracle().orc_default_evalue()  # 1/powl(10,20) evaluated in long double (src/IMSAME.c:44)
     else:
         p.min_e_value = float(evalue)
     p.min_coverage = float(coverage)
@@ -94,25 +96,6 @@ def default_params(n_threads=4, evalue=None, coverage=0.5, identity=0.5, igap=5,
     p.k = k  # 12 = FIXED_K (src/structs.h:15), the only value the reference itself can pin
     p.db_total_len_global = db_total_len_global
     return p
-
-
-_ld_helper = None
-
-
-def _ld_default_evalue():
-    """1/powl(10,20) evaluated in long double (src/IMSAME.c:44) -- via a tiny C helper."""
-    global _ld_helper
-    if _ld_helper is None:
-        src = os.path.join(ROOT, "oracle", "_build", "ldhelper.c")
-        so = os.path.join(ROOT, "oracle", "_build", "ldhelper.so")
-        os.makedirs(os.path.dirname(src), exist_ok=True)
-        if not os.path.exists(so):
-            with open(src, "w") as f:
-                f.write("#include <math.h>\nlong double imsame_default_evalue(void){return 1/powl(10,20);}\n")
-            subprocess.check_call(["gcc", "-O2", "-shared", "-fPIC", src, "-lm", "-o", so])
-        _ld_helper = C.CDLL(so)
-        _ld_helper.imsame_default_evalue.restype = C.c_longdouble
-    return _ld_helper.imsame_default_evalue()
 
 
 class OracleSeqs:
@@ -238,6 +221,38 @@ def split_align_records(path):
 
 def have_reference():
     return os.path.exists(REF_BIN)
+
+
+PINS = os.path.join(ROOT, "tests", "golden", "reference_pins.json")
+_pins = None
+
+
+def pins(section):
+    """what the reference tools gave on the seeded inputs of the tests that compare with them (see the file's "about")"""
+    global _pins
+    if _pins is None:
+        import json
+        with open(PINS) as f:
+            _pins = json.load(f)
+    return _pins[section]
+
+
+def sha(data):
+    import hashlib
+    return hashlib.sha256(data).hexdigest()
+
+
+def align_digest(path, whole=False, lines=False):
+    """the parts of a .align file the reference comparisons look at: record count, sorted header lines, the sorted
+    lines of the whole file (lines=True), the bytes (whole=True: -n_threads 1 output)"""
+    data = open(path, "rb").read()
+    d = {"records": len(parse_align_headers(path)),
+         "headers": sha(b"\n".join(sorted(l for l in data.split(b"\n") if HEADER_RE.match(l))))}
+    if lines:
+        d["sorted_lines"] = sha(b"\n".join(sorted(data.split(b"\n"))))
+    if whole:
+        d["bytes"] = sha(data)
+    return d
 
 
 def run_reference(query_fa, db_fa, out_path, n_threads=4, extra=()):

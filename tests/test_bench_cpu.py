@@ -58,6 +58,45 @@ def test_sampled_parity_accepts_right_records_and_sees_every_field(built):
     assert b.sampled_parity(nq, bad, *args)["mismatches"] == 1
 
 
+def test_dump_records_writes_every_field_exactly_and_samples_above_the_cap(built, tmp_path):
+    b = _bench()
+    rng = np.random.default_rng(4)
+    n = 5000
+    rec = np.zeros(n, dtype=REC)
+    rec["accepted"] = rng.integers(0, 2, n)
+    rec["db_seq"] = rng.integers(0, 80_000_000, n)
+    rec["qpos_end"] = rng.integers(0, 250_000_000, n)
+    rec["db_pos"] = rng.integers(0, 20_000_000_000, n)
+    rec["length"] = rng.integers(0, 3000, n)
+    rec["identities"] = rng.integers(0, 3000, n)
+    b.dump_records(str(tmp_path / "all"), rec, np)
+    got = {f[:-4]: np.load(tmp_path / "all" / f) for f in os.listdir(tmp_path / "all")}
+    assert sorted(got) == sorted(["read"] + [f for f, _ in b.DUMP_FIELDS])
+    assert all(v.dtype in (np.float32, np.float64) and len(v) == n for v in got.values())
+    assert np.array_equal(got["read"], np.arange(n))
+    for f, _ in b.DUMP_FIELDS:
+        assert np.array_equal(got[f].astype(np.uint64), rec[f].astype(np.uint64)), f
+    b.DUMP_BYTES_MAX = 1000 * 44  # 44 bytes per read: a fixed sample of 1000 reads
+    for d in ("s1", "s2"):
+        b.dump_records(str(tmp_path / d), rec, np)
+    assert sum(os.path.getsize(tmp_path / "s1" / f) - 128 for f in os.listdir(tmp_path / "s1")) == b.DUMP_BYTES_MAX
+    reads = np.load(tmp_path / "s1" / "read.npy").astype(np.int64)
+    assert len(reads) == 1000 and np.array_equal(reads, np.load(tmp_path / "s2" / "read.npy"))
+    assert np.array_equal(np.load(tmp_path / "s1" / "db_pos.npy"), rec["db_pos"][reads].astype(np.float64))
+
+
+def test_zero_timed_steps_is_refused(tmp_path):
+    r = subprocess.run([sys.executable, os.path.join(hp.ROOT, "bench.py"), "--steps", "0"], capture_output=True, text=True,
+                       timeout=120, cwd=str(tmp_path))
+    assert r.returncode == 2 and "--steps must be at least 1" in r.stderr and not r.stdout
+
+
+def test_dump_outputs_is_refused_on_the_reference_arm(tmp_path):
+    r = subprocess.run([sys.executable, os.path.join(hp.ROOT, "bench.py"), "--impl", "reference", "--dump-outputs",
+                        str(tmp_path / "d")], capture_output=True, text=True, timeout=120, cwd=str(tmp_path))
+    assert r.returncode == 2 and "not with --impl reference" in r.stderr and not os.path.exists(tmp_path / "d")
+
+
 @pytest.mark.skipif(not hp.have_reference(), reason="oracle/_ref not built (needs /root/reference at build time)")
 def test_reference_arm_prints_the_contract_line(built, tmp_path):
     r = subprocess.run([sys.executable, os.path.join(hp.ROOT, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "1",

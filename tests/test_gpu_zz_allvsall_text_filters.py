@@ -48,6 +48,10 @@ def test_all_vs_all_with_samples_that_are_not_their_mirror(gpu, tmp_path):
     # the reverse-strand samples match the forward one through their reverse complement
     for n in ("s0-s1.r.align", "s0-s2.r.align", "s0-s3.r.align"):
         assert os.path.getsize(o2 / n) > 5000, n
+    # the query-s0 files against what the reference workflow wrote (tests/golden/reference_pins.json)
+    want = hp.pins("allvsall_text_filter_samples")
+    for n in want:
+        assert hp.align_digest(str(o2 / n), lines=True) == want[n], n
     ref_script = os.path.join(hp.ROOT, "oracle", "_ref", "all_vs_all_metagenomes_IMSAME.sh")
     if os.path.exists(ref_script) and hp.have_reference():
         subprocess.run(["bash", ref_script] + args + [str(o3)], stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)

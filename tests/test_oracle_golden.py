@@ -57,24 +57,37 @@ def test_bulk_min_key_form_equals_scan_order(name, n_threads):
     assert len(hp.best_to_records(a, nq)) > (5 if nq > 5 else 1)
 
 
-@pytest.mark.skipif(not hp.have_reference(), reason="oracle/_ref/IMSAME not built (no /root/reference here)")
-@pytest.mark.parametrize("seed,div,n_threads", [(1001, 0.03, 1), (7, 0.10, 4), (99, 0.20, 8)])
-def test_oracle_vs_live_reference(seed, div, n_threads, tmp_path):
-    """fresh seeded inputs through the real reference binary"""
+LIVE_CASES = [(1001, 0.03, 1), (7, 0.10, 4), (99, 0.20, 8)]
+
+
+def live_case(seed, div, n_threads, d):
+    """seeded inputs of test_oracle_vs_live_reference and the oracle's .align file on them"""
     from imsame_b200 import hostlib as H
     pool = H.SynthPool(seed, 3, 60000)
     nd, nq, L = 6000, 600, 150
-    dbf, qf, ref_out, orc_out = (str(tmp_path / n) for n in ("db.fa", "q.fa", "ref.align", "orc.align"))
+    dbf, qf, orc_out = (os.path.join(d, n) for n in ("db.fa", "q.fa", "orc.align"))
     H.write_fasta(dbf, pool.db_reads(0, nd, L), nd, L, "d")
     H.write_fasta(qf, pool.query_reads(0, nq, L, div), nq, L, "q")
     pool.close()
-    hp.run_reference(qf, dbf, ref_out, n_threads=n_threads)
     db, q = hp.OracleSeqs(dbf, True), hp.OracleSeqs(qf, False)
     hp.oracle_align(db, q, hp.default_params(n_threads=n_threads), out_path=orc_out)
-    if n_threads == 1:
-        assert open(ref_out, "rb").read() == open(orc_out, "rb").read()
-    assert hp.parse_align_headers(ref_out) == hp.parse_align_headers(orc_out)
-    assert len(hp.parse_align_headers(ref_out)) > 100
+    return dbf, qf, orc_out
+
+
+@pytest.mark.parametrize("seed,div,n_threads", LIVE_CASES)
+def test_oracle_vs_live_reference(seed, div, n_threads, tmp_path):
+    """fresh seeded inputs through the real reference binary where oracle/_ref is built; its output on them is
+    pinned in tests/golden/reference_pins.json"""
+    dbf, qf, orc_out = live_case(seed, div, n_threads, str(tmp_path))
+    if hp.have_reference():
+        ref_out = str(tmp_path / "ref.align")
+        hp.run_reference(qf, dbf, ref_out, n_threads=n_threads)
+        if n_threads == 1:
+            assert open(ref_out, "rb").read() == open(orc_out, "rb").read()
+        assert hp.parse_align_headers(ref_out) == hp.parse_align_headers(orc_out)
+    got = hp.align_digest(orc_out, whole=n_threads == 1)
+    assert got == hp.pins("oracle_vs_live_reference")[f"{seed}/{div}/{n_threads}"]
+    assert got["records"] > 100
 
 
 @pytest.mark.parametrize("k", [8, 10, 14])
