@@ -64,6 +64,7 @@ SYMBOLS = ["imsame_gpu_create", "imsame_gpu_destroy", "imsame_gpu_strerror", "im
            "imsame_gpu_mask_payload", "imsame_gpu_fetch", "imsame_gpu_nw_batch", "imsame_gpu_set_nw_mode", "imsame_gpu_set_passes",
            "imsame_gpu_set_kmer", "imsame_gpu_comm_id", "imsame_gpu_comm_init", "imsame_gpu_comm_free",
            "imsame_gpu_run_sharded", "imsame_gpu_align_shard", "imsame_gpu_align_sharded",
+           "imsame_gpu_db_revcomp", "imsame_gpu_align_revcomp",
            "imsame_gpu_sample_create", "imsame_gpu_sample_revcomp", "imsame_gpu_sample_free", "imsame_gpu_align_samples",
            "imsame_gpu_traceback", "imsame_gpu_free", "imsame_gpu_host_alloc", "imsame_gpu_host_free"]
 
@@ -120,6 +121,8 @@ def lib():
         l.imsame_gpu_align_shard.argtypes = [vp, C.POINTER(SeqInfo), C.POINTER(SeqInfo), C.POINTER(Params), vp, vp, C.POINTER(Stats)]
         l.imsame_gpu_align_sharded.argtypes = [C.POINTER(vp), C.c_int, C.POINTER(SeqInfo), C.POINTER(SeqInfo),
                                                C.POINTER(Params), vp, C.POINTER(Stats)]
+        l.imsame_gpu_db_revcomp.argtypes = [vp]
+        l.imsame_gpu_align_revcomp.argtypes = [C.POINTER(vp), C.c_int, vp, C.POINTER(Stats)]
         l.imsame_gpu_sample_create.argtypes = [vp, C.POINTER(SeqInfo), C.POINTER(vp)]
         l.imsame_gpu_sample_revcomp.argtypes = [vp, vp, C.POINTER(vp)]
         l.imsame_gpu_sample_free.argtypes = [vp, vp]
@@ -295,6 +298,18 @@ class Imsame:
         self._check(L.imsame_gpu_run_end(self._h, C.byref(st)))
         return st.as_dict()
 
+    # -- the reverse strand of the resident database
+    def db_revcomp(self):
+        """the resident database becomes its reverse complement (reads in reverse order, each reverse complemented:
+        what revComp writes); a second call restores it"""
+        self._check(lib().imsame_gpu_db_revcomp(self._h))
+
+    def align_revcomp(self):
+        """the query and parameters of the previous align(), against the reverse complement of its database, which is
+        still resident.  Returns (records, stats) like align(); db_seq / db_pos count in the reverse database."""
+        out, st = align_revcomp([self])
+        return out, st[0]
+
     # -- read sets resident on the device (all-vs-all)
     def sample(self, reads, breaks=None):
         """upload + pack once; returns a handle usable as database or query of align_samples"""
@@ -434,6 +449,19 @@ def align_sharded(ctxs, db, query, params=None, db_breaks=None):
         raise ImsameError(rc, lib().imsame_gpu_last_cuda_error(ctxs[0]._h).decode())
     for c in ctxs:
         c.nq = int(q.n_seqs)
+    return out, [s.as_dict() for s in st]
+
+
+def align_revcomp(ctxs):
+    """one process, len(ctxs) GPUs: the previous align_sharded() (or, one context, align()) again, against the reverse
+    complement of its database, still resident on the same contexts.  Returns (records, [stats per shard])."""
+    n = len(ctxs)
+    out = np.zeros(ctxs[0].nq, dtype=BEST_DTYPE)
+    hs = (C.c_void_p * n)(*[c._h for c in ctxs])
+    st = (Stats * n)()
+    rc = lib().imsame_gpu_align_revcomp(hs, n, out.ctypes.data, st)
+    if rc:
+        raise ImsameError(rc, lib().imsame_gpu_last_cuda_error(ctxs[0]._h).decode())
     return out, [s.as_dict() for s in st]
 
 

@@ -17,6 +17,7 @@
 #include "nw.cuh"
 #include "nwp_launch.h"
 #include "qtable.cuh"
+#include "revcomp.cuh"
 #include "scan.cuh"
 
 using namespace imsame;
@@ -83,6 +84,11 @@ struct imsame_ctx {
     uint64_t db_total = 0, db_nseqs = 0;
     uint32_t db_maxlen = 0;
     bool have_db = false;
+    bool db_rc = false;  // the resident database is the reverse complement of what was uploaded (imsame_gpu_db_revcomp)
+    // the query and database of the last successful imsame_gpu_align (1) / imsame_gpu_align_sharded over this many
+    // contexts, still resident, and the parameters this context ran it with (imsame_gpu_align_revcomp); 0 = none
+    int last_align = 0;
+    imsame_params align_params;
 
     // tables + work buffers
     uint16_t *d_nmin = nullptr, *d_lmin = nullptr, *d_imin = nullptr;
@@ -270,6 +276,7 @@ void free_query(imsame_ctx *ctx) {
     pool_free(ctx, ctx->qtab_early); pool_free(ctx, ctx->qtab_late);
     ctx->tab_full = ctx->tab_early = false;
     ctx->have_query = false;
+    ctx->last_align = 0;
 }
 void free_db(imsame_ctx *ctx) {
     for (Seg &s : ctx->segs) {
@@ -278,6 +285,8 @@ void free_db(imsame_ctx *ctx) {
     }
     ctx->segs.clear();
     ctx->have_db = false;
+    ctx->db_rc = false;
+    ctx->last_align = 0;
 }
 
 uint32_t uniform_len(const uint64_t *start, uint64_t n, uint64_t total) {
@@ -1447,6 +1456,8 @@ int imsame_gpu_align(imsame_ctx *ctx, const imsame_seqinfo *db, const imsame_seq
     cudaStreamSynchronize(ctx->copy_stream);
     for (Seg &s : ctx->segs) s.wait_ready = false;
     if (rc) { ctx->have_db = false; return rc; }
+    ctx->last_align = 1;
+    ctx->align_params = *p;
     const double t3 = now();
     if ((rc = imsame_gpu_fetch(ctx, nullptr, nullptr, out))) return rc;
     if (trace) fprintf(stderr, "[imsame] host wall ms: upload + table + scan + NW %.1f  fetch %.1f\n", t3 - t0, now() - t3);

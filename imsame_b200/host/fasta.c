@@ -355,6 +355,28 @@ int imsame_revcomp_is_mirror(const imsame_fasta *fwd, const imsame_fasta *rev) {
     return !differ;
 }
 
+/* The in-memory form of `revComp path r.fa` + the database loader: the file mapped, reverse complemented
+ * (imsame_revcomp_mem) and parsed with is_db = 1.  *has_u: the file holds a 'U' or 'u'. */
+int imsame_revcomp_load(const char *path, imsame_fasta *rev, int *has_u) {
+    memset(rev, 0, sizeof(*rev));
+    imsame_file_image img;
+    if (imsame_file_map(path, &img)) return 1;
+    *has_u = memchr(img.data, 'U', img.len) != NULL || memchr(img.data, 'u', img.len) != NULL;
+    unsigned char *rc = NULL;
+    size_t rc_len = 0;
+    const int e = imsame_revcomp_mem(img.data, img.len, &rc, &rc_len);
+    imsame_file_unmap(&img);
+    if (e) return 2;
+    const int pe = imsame_fasta_parse_mem(rc, rc_len, 1, rev);
+    free(rc);
+    return pe ? 3 : 0;
+}
+
+/* revComp turns U into an A the loader keeps, so a file with a U never qualifies, whatever the parses say */
+int imsame_revcomp_on_device(const imsame_fasta *fwd, const imsame_fasta *rev, int has_u) {
+    return !has_u && imsame_revcomp_is_mirror(fwd, rev);
+}
+
 void imsame_fasta_free(imsame_fasta *f) {
     free(f->sequences);
     free(f->start_pos);

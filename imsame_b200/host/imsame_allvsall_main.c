@@ -43,8 +43,7 @@ typedef struct {
     imsame_fasta fwd, rev; /* parsed forward sample / parsed revComp(sample): what the records are rendered from */
     int have_fwd, have_rev;
     imsame_sample *dfwd, *drev; /* the same two read sets resident on the device */
-    int has_u;                  /* the file contains a 'U': revComp turns it into an 'A' the loader keeps, so the
-                                   reverse complement has to be uploaded from the text form */
+    int has_u;                  /* the file contains a 'U' (imsame_revcomp_load, imsame_revcomp_on_device) */
 } sample;
 
 static int by_name(const void *a, const void *b) { return strcoll(((const sample *)a)->name, ((const sample *)b)->name); }
@@ -66,15 +65,11 @@ static void need_reverse(sample *s, const char *dir, const char *ext) {
     if (s->have_rev) return;
     char path[4096];
     snprintf(path, sizeof path, "%s/%s.%s", dir, s->name, ext);
-    imsame_file_image img;
-    if (imsame_file_map(path, &img)) terror("opening IN sequence FASTA file");
-    s->has_u = memchr(img.data, 'U', img.len) != NULL || memchr(img.data, 'u', img.len) != NULL;
-    unsigned char *rc = NULL;
-    size_t rc_len = 0;
-    if (imsame_revcomp_mem(img.data, img.len, &rc, &rc_len)) terror("memory for Seq");
-    imsame_file_unmap(&img);
-    if (imsame_fasta_parse_mem(rc, rc_len, 1, &s->rev)) terror("Could not allocate memory for database vector");
-    free(rc);
+    switch (imsame_revcomp_load(path, &s->rev, &s->has_u)) {
+        case 1: terror("opening IN sequence FASTA file");
+        case 2: terror("memory for Seq");
+        case 3: terror("Could not allocate memory for database vector");
+    }
     s->have_rev = 1;
 }
 
@@ -100,8 +95,7 @@ static void need_reverse_dev(sample *s, imsame_ctx *ctx) {
        not the loader's (imsame_revcomp_is_mirror, host/fasta.c: '\r' / '-' / digits inside a record, 'U', header lines
        with several '>').  Both parses are in memory for the renderer anyway: the device path is taken only when
        the parse of revComp's text IS the mirror image of the sample, otherwise that parse is uploaded. */
-    const int same_shape = s->have_fwd && s->have_rev && imsame_revcomp_is_mirror(&s->fwd, &s->rev);
-    if (s->has_u || !s->have_fwd || !same_shape) {
+    if (!(s->have_fwd && s->have_rev && imsame_revcomp_on_device(&s->fwd, &s->rev, s->has_u))) {
         imsame_seqinfo v;
         imsame_fasta_view(&s->rev, &v);
         rc = imsame_gpu_sample_create(ctx, &v, &s->drev);

@@ -39,6 +39,13 @@ void imsame_file_unmap(imsame_file_image *img);
 int imsame_revcomp_mem(const unsigned char *buf, size_t n, unsigned char **out, size_t *out_len);
 /* 1 when `rev` (parse of revComp's output) is exactly the mirror image of `fwd`: bases, read offsets, word breaks */
 int imsame_revcomp_is_mirror(const imsame_fasta *fwd, const imsame_fasta *rev);
+/* revComp(path) as the database loader sees it (`revComp path r.fa` + imsame_fasta_load(r.fa, 1), in memory): 0, or
+ * 1 = the file could not be read, 2 = no memory for its reverse complement, 3 = none for the parse.  *has_u: the
+ * file holds a 'U' or 'u'.  Then imsame_revcomp_on_device(fwd, rev, has_u) decides whether the device may derive the
+ * reverse read set from the forward one (imsame_gpu_sample_revcomp, imsame_gpu_db_revcomp) or has to upload rev:
+ * rev is the mirror image of fwd and the file had no U (which revComp turns into an A the loader keeps). */
+int imsame_revcomp_load(const char *path, imsame_fasta *rev, int *has_u);
+int imsame_revcomp_on_device(const imsame_fasta *fwd, const imsame_fasta *rev, int has_u);
 void imsame_fasta_free(imsame_fasta *f);
 void imsame_fasta_view(const imsame_fasta *f, imsame_seqinfo *v);
 

@@ -30,6 +30,112 @@ static void *ctx_main(void *arg) {
     return NULL;
 }
 
+/* traceback on the GPU + rendering of the records of the accepted reads of `best` (db: what best[].db_seq indexes) */
+static int write_records(imsame_ctx **ctx, const imsame_job_opts *o, const imsame_fasta *qf, const imsame_fasta *dbf,
+                         const imsame_params *p, const imsame_best *best, FILE *fout, char *err, size_t errlen, double *tp) {
+    const imsame_fasta q = *qf, db = *dbf;
+    imsame_seqinfo qv, dv;
+    imsame_fasta_view(&q, &qv);
+    imsame_fasta_view(&db, &dv);
+    int rc = IMSAME_OK;
+    if (!*ctx && (rc = imsame_gpu_create(ctx, o->device))) return rc;
+    uint64_t *ops_off = (uint64_t *)malloc((q.n_seqs + 1) * sizeof(uint64_t));
+    uint32_t *cell = (uint32_t *)malloc(4 * q.n_seqs * sizeof(uint32_t)), *ops = NULL;
+    rc = (ops_off && cell) ? imsame_gpu_traceback(*ctx, &dv, &qv, p, best, ops_off, &ops, cell) : IMSAME_ENOMEM;
+    if (rc) {
+        if (err && errlen) snprintf(err, errlen, "%s", imsame_gpu_last_cuda_error(*ctx));
+    } else {
+        if (o->trace) { fprintf(stderr, "[imsame] traceback (GPU) %.3f s\n", now_s() - *tp); *tp = now_s(); }
+        /* records are rendered by all host threads, each into its own buffer for a contiguous range of
+           reads, and written in ascending read order (the reference's order with -n_threads 1) */
+        int nt = 1;
+#ifdef _OPENMP
+        nt = omp_get_max_threads();
+#endif
+        if (nt > 64) nt = 64;
+        if ((uint64_t)nt > q.n_seqs) nt = (int)q.n_seqs;
+        char *bufs[64];
+        size_t lens[64];
+        int failed = 0;
+        memset(bufs, 0, sizeof bufs);
+        memset(lens, 0, sizeof lens);
+#pragma omp parallel for schedule(static, 1) num_threads(nt)
+        for (int t = 0; t < nt; t++) {
+            const uint64_t r0 = q.n_seqs * (uint64_t)t / (uint64_t)nt, r1 = q.n_seqs * (uint64_t)(t + 1) / (uint64_t)nt;
+            const size_t rec_max = 6 * (2 * (size_t)IMSAME_MAX_READ_SIZE) + 768;
+            size_t cap = 1 << 20, len = 0;
+            char *buf = (char *)malloc(cap);
+            for (uint64_t r = r0; r < r1 && buf; r++) {
+                if (!best[r].accepted) continue;
+                if (cap - len < rec_max) {
+                    cap = cap * 2 + rec_max;
+                    char *nb2 = (char *)realloc(buf, cap);
+                    if (!nb2) { free(buf); buf = NULL; break; }
+                    buf = nb2;
+                }
+                const uint64_t s = best[r].db_seq;
+                const uint32_t xlen = (uint32_t)(db.start_pos[s + 1] - db.start_pos[s]);
+                const uint32_t ylen = (uint32_t)(q.start_pos[r + 1] - q.start_pos[r]);
+                len += (size_t)imsame_format_header(buf + len, r, s, best[r].length, best[r].identities, ylen);
+                len += (size_t)imsame_render_alignment(buf + len, db.sequences + db.start_pos[s], xlen,
+                                                       q.sequences + q.start_pos[r], ylen, cell[4 * r], cell[4 * r + 1],
+                                                       ops + ops_off[r], ops_off[r + 1] - ops_off[r]);
+            }
+            if (!buf) {
+#pragma omp atomic write
+                failed = 1;
+            }
+            bufs[t] = buf;
+            lens[t] = len;
+        }
+        for (int t = 0; t < nt; t++) {
+            if (!failed && bufs[t]) fwrite(bufs[t], 1, lens[t], fout);
+            free(bufs[t]);
+        }
+        if (failed) rc = IMSAME_ENOMEM;
+        if (o->trace) { fprintf(stderr, "[imsame] render + write %.3f s\n", now_s() - *tp); *tp = now_s(); }
+    }
+    imsame_gpu_free(ops);
+    free(ops_off);
+    free(cell);
+    return rc;
+}
+
+/* the reverse strand (o->rev) on the contexts of the forward one: ctxs[0 .. ng) (ctxs == &ctx when ng == 1) */
+static int reverse_strand(imsame_ctx **ctxs, int ng, const imsame_job_opts *o, const imsame_fasta *q, imsame_params *p,
+                          char *err, size_t errlen, double *tp) {
+    imsame_rev_job *rv = o->rev;
+    int on_device = 0;
+    const imsame_fasta *rdb = rv->wait(rv->arg, &on_device);
+    if (!rdb) return IMSAME_EARG;
+    if (o->trace) { fprintf(stderr, "[imsame] reverse strand ready (%s) %.3f s\n", on_device ? "device" : "upload", now_s() - *tp); *tp = now_s(); }
+    if (rdb->n_seqs == 0) return IMSAME_OK;
+    imsame_best *best = (imsame_best *)calloc(q->n_seqs, sizeof(imsame_best));
+    if (!best) return IMSAME_ENOMEM;
+    imsame_seqinfo qv, rv_view;
+    imsame_fasta_view(q, &qv);
+    imsame_fasta_view(rdb, &rv_view);
+    int rc;
+    if (on_device) {  /* the forward database is still resident: mirrored there (rdb has its shape) */
+        rc = imsame_gpu_align_revcomp(ctxs, ng, best, NULL);
+    } else {          /* revComp's text parses into something else: upload that parse, as a second process would */
+        int nr = ng;
+        if ((uint64_t)nr > rdb->n_seqs) nr = (int)rdb->n_seqs;
+        rc = nr == 1 ? imsame_gpu_align(ctxs[0], &rv_view, &qv, p, best, NULL)
+                     : imsame_gpu_align_sharded(ctxs, nr, &rv_view, &qv, p, best, NULL);
+    }
+    if (rc && err && errlen) snprintf(err, errlen, "%s", imsame_gpu_last_cuda_error(ctxs[0]));
+    if (o->trace) { fprintf(stderr, "[imsame] align reverse strand %.3f s\n", now_s() - *tp); *tp = now_s(); }
+    uint64_t accepted = 0;
+    if (!rc) {
+        for (uint64_t r = 0; r < q->n_seqs; r++) accepted += best[r].accepted;
+        if (rv->out != NULL && accepted > 0) rc = write_records(&ctxs[0], o, q, rdb, p, best, rv->out, err, errlen, tp);
+    }
+    rv->accepted = accepted;
+    free(best);
+    return rc;
+}
+
 int imsame_run_job(const imsame_fasta *qf, const imsame_fasta *dbf, const imsame_job_opts *o, FILE *fout,
                    imsame_ctx **ctx_cache, uint64_t *accepted_out, char *err, size_t errlen) {
     const imsame_fasta q = *qf, db = *dbf;
@@ -56,6 +162,7 @@ int imsame_run_job(const imsame_fasta *qf, const imsame_fasta *dbf, const imsame
     int ng = o->gpus < 1 ? 1 : o->gpus;
     if ((uint64_t)ng > db.n_seqs) ng = (int)db.n_seqs;
     imsame_ctx *ctx = NULL; /* device `o->device`: alignment (shard 0) and traceback; kept if the caller caches */
+    imsame_ctx **ctxs = NULL; /* ng > 1: the shards' contexts, kept until the reverse strand is done (o->rev) */
     int rc = IMSAME_OK;
     if (ctx_cache && *ctx_cache) ctx = *ctx_cache;
     if (ng == 1) {
@@ -72,7 +179,7 @@ int imsame_run_job(const imsame_fasta *qf, const imsame_fasta *dbf, const imsame
            reduced with NCCL inside the library (imsame_gpu_align_sharded), replacing src/IMSAME.c:430-467 */
         ctx_job *jobs = (ctx_job *)calloc((size_t)ng, sizeof(ctx_job));
         pthread_t *th = (pthread_t *)calloc((size_t)ng, sizeof(pthread_t));
-        imsame_ctx **ctxs = (imsame_ctx **)calloc((size_t)ng, sizeof(imsame_ctx *));
+        ctxs = (imsame_ctx **)calloc((size_t)ng, sizeof(imsame_ctx *));
         if (!jobs || !th || !ctxs) {
             free(jobs); free(th); free(ctxs); free(best);
             return IMSAME_ENOMEM;
@@ -96,78 +203,29 @@ int imsame_run_job(const imsame_fasta *qf, const imsame_fasta *dbf, const imsame
             rc = imsame_gpu_align_sharded(ctxs, ng, &dv, &qv, &p, best, NULL);
             if (rc && err && errlen) snprintf(err, errlen, "%s", imsame_gpu_last_cuda_error(ctxs[0]));
         }
-        for (int g = 1; g < ng; g++) imsame_gpu_destroy(ctxs[g]);
+        if (!o->rev || rc)
+            for (int g = 1; g < ng; g++) imsame_gpu_destroy(ctxs[g]);
         ctx = ctxs[0];
         if (ctx_cache && ctx) *ctx_cache = ctx;
         free(jobs);
         free(th);
-        free(ctxs);
+        if (!o->rev || rc) { free(ctxs); ctxs = NULL; }
     }
     if (rc) { free(best); if (ctx && !(ctx_cache && *ctx_cache == ctx)) imsame_gpu_destroy(ctx); return rc; }
     for (uint64_t r = 0; r < q.n_seqs; r++) accepted += best[r].accepted;
     if (o->trace) { fprintf(stderr, "[imsame] align (all shards) %.3f s\n", now_s() - tp); tp = now_s(); }
 
-    if (fout != NULL && accepted > 0) {
-        if (!ctx && (rc = imsame_gpu_create(&ctx, o->device))) { free(best); return rc; }
-        uint64_t *ops_off = (uint64_t *)malloc((q.n_seqs + 1) * sizeof(uint64_t));
-        uint32_t *cell = (uint32_t *)malloc(4 * q.n_seqs * sizeof(uint32_t)), *ops = NULL;
-        rc = (ops_off && cell) ? imsame_gpu_traceback(ctx, &dv, &qv, &p, best, ops_off, &ops, cell) : IMSAME_ENOMEM;
-        if (rc) {
-            if (err && errlen) snprintf(err, errlen, "%s", imsame_gpu_last_cuda_error(ctx));
-        } else {
-            if (o->trace) { fprintf(stderr, "[imsame] traceback (GPU) %.3f s\n", now_s() - tp); tp = now_s(); }
-            /* records are rendered by all host threads, each into its own buffer for a contiguous range of
-               reads, and written in ascending read order (the reference's order with -n_threads 1) */
-            int nt = 1;
-#ifdef _OPENMP
-            nt = omp_get_max_threads();
-#endif
-            if (nt > 64) nt = 64;
-            if ((uint64_t)nt > q.n_seqs) nt = (int)q.n_seqs;
-            char *bufs[64];
-            size_t lens[64];
-            int failed = 0;
-            memset(bufs, 0, sizeof bufs);
-            memset(lens, 0, sizeof lens);
-#pragma omp parallel for schedule(static, 1) num_threads(nt)
-            for (int t = 0; t < nt; t++) {
-                const uint64_t r0 = q.n_seqs * (uint64_t)t / (uint64_t)nt, r1 = q.n_seqs * (uint64_t)(t + 1) / (uint64_t)nt;
-                const size_t rec_max = 6 * (2 * (size_t)IMSAME_MAX_READ_SIZE) + 768;
-                size_t cap = 1 << 20, len = 0;
-                char *buf = (char *)malloc(cap);
-                for (uint64_t r = r0; r < r1 && buf; r++) {
-                    if (!best[r].accepted) continue;
-                    if (cap - len < rec_max) {
-                        cap = cap * 2 + rec_max;
-                        char *nb2 = (char *)realloc(buf, cap);
-                        if (!nb2) { free(buf); buf = NULL; break; }
-                        buf = nb2;
-                    }
-                    const uint64_t s = best[r].db_seq;
-                    const uint32_t xlen = (uint32_t)(db.start_pos[s + 1] - db.start_pos[s]);
-                    const uint32_t ylen = (uint32_t)(q.start_pos[r + 1] - q.start_pos[r]);
-                    len += (size_t)imsame_format_header(buf + len, r, s, best[r].length, best[r].identities, ylen);
-                    len += (size_t)imsame_render_alignment(buf + len, db.sequences + db.start_pos[s], xlen,
-                                                           q.sequences + q.start_pos[r], ylen, cell[4 * r], cell[4 * r + 1],
-                                                           ops + ops_off[r], ops_off[r + 1] - ops_off[r]);
-                }
-                if (!buf) {
-#pragma omp atomic write
-                    failed = 1;
-                }
-                bufs[t] = buf;
-                lens[t] = len;
-            }
-            for (int t = 0; t < nt; t++) {
-                if (!failed && bufs[t]) fwrite(bufs[t], 1, lens[t], fout);
-                free(bufs[t]);
-            }
-            if (failed) rc = IMSAME_ENOMEM;
-            if (o->trace) { fprintf(stderr, "[imsame] render + write %.3f s\n", now_s() - tp); tp = now_s(); }
-        }
-        imsame_gpu_free(ops);
-        free(ops_off);
-        free(cell);
+    if (fout != NULL && accepted > 0) rc = write_records(&ctx, o, &q, &db, &p, best, fout, err, errlen, &tp);
+    if (!rc && o->rev) {
+        /* the forward records are complete: a read-size stop of the reverse strand leaves them as the first process
+           of the two-process workflow would */
+        if (ctxs) ctxs[0] = ctx;
+        o->rev->rc = reverse_strand(ctxs ? ctxs : &ctx, ng, o, &q, &p, err, errlen, &tp);
+        if (ctxs) ctx = ctxs[0];
+    }
+    if (ctxs) {
+        for (int g = 1; g < ng; g++) imsame_gpu_destroy(ctxs[g]);
+        free(ctxs);
     }
     if (ctx && !(ctx_cache && *ctx_cache == ctx)) imsame_gpu_destroy(ctx);
     free(best);

@@ -9,6 +9,19 @@
 #define IMSAME_JOB_H
 #include "imsame_host.h"
 
+/* The reverse strand in the same job (IMSAME -out_rev): the records of `IMSAME -db revComp(db)` against the
+ * database still resident on the job's GPU(s) where the mirror rule holds (imsame_revcomp_on_device), else against
+ * an upload of the reverse parse. */
+typedef struct imsame_rev_job {
+    FILE *out; /* its records */
+    /* called once the forward records are written: the parse of revComp(db) (imsame_revcomp_load) with
+       *on_device = imsame_revcomp_on_device(db, rev, has_u), or NULL when it could not be built */
+    const imsame_fasta *(*wait)(void *arg, int *on_device);
+    void *arg;
+    uint64_t accepted; /* out: reads with a record against the reverse complement */
+    int rc;            /* out: the reverse strand's result (the job returns the forward strand's) */
+} imsame_rev_job;
+
 typedef struct imsame_job_opts {
     uint64_t n_threads;
     long double minevalue, mincoverage, minidentity;
@@ -20,10 +33,12 @@ typedef struct imsame_job_opts {
        copies q / db are still what the records are rendered from */
     imsame_sample *q_sample;
     const imsame_sample *db_sample;
+    /* optional (not with the samples): the reverse strand too, after the forward records are written */
+    imsame_rev_job *rev;
 } imsame_job_opts;
 
 /* Aligns every read of q against db and writes the records of the accepted reads to fout (may be
- * NULL: only count).  *ctx_cache (may be NULL) keeps the context of `device` alive between jobs when
+ * NULL: only count); then, with o->rev, the same against revComp(db) into o->rev->out.  *ctx_cache (may be NULL) keeps the context of `device` alive between jobs when
  * gpus == 1.  Returns 0 or an IMSAME_E* code; err receives the CUDA detail. */
 int imsame_run_job(const imsame_fasta *q, const imsame_fasta *db, const imsame_job_opts *o, FILE *fout,
                    imsame_ctx **ctx_cache, uint64_t *accepted, char *err, size_t errlen);

@@ -16,6 +16,13 @@
  *   -gpus N     shard the database by contiguous read ranges over N GPUs (default 1)
  *   -kmer K     seed length 4..16 (default 12 = the reference's FIXED_K; it has no such flag)
  *   -device D   first CUDA device to use (default 0)
+ *   -out_rev F  also align the query against the reverse complement of the database and write those records to F:
+ *               what `revComp db db.r; IMSAME ... -db db.r -out F` writes, in the same run.  The reverse read set is
+ *               built by a host thread while the forward strand runs; where it is the mirror image of the database
+ *               (imsame_revcomp_on_device) the database already on the GPU(s) is reverse complemented in place
+ *               (imsame_gpu_align_revcomp), otherwise the reverse parse is uploaded.  stdout gains two lines after
+ *               the Jaccard index, the numbers the second process would print; -out is what the run without the
+ *               flag writes.  (Not in --help, whose text is the reference's.)
  */
 #define _GNU_SOURCE
 #include <inttypes.h>
@@ -42,7 +49,7 @@ static double now_s(void) {
 }
 
 typedef struct {
-    const char *query, *db, *out;
+    const char *query, *db, *out, *out_rev;
     uint64_t n_threads;
     long double minevalue, mincoverage, minidentity;
     int igap, egap;
@@ -67,7 +74,7 @@ static void usage_and_exit(void) { /* src/IMSAME.c:526-538 */
 
 static void parse_args(int argc, char **av, cli_args *a) {
     /* defaults: src/IMSAME.c:44-49 */
-    a->query = a->db = a->out = NULL;
+    a->query = a->db = a->out = a->out_rev = NULL;
     a->n_threads = 4;
     a->minevalue = 1 / powl(10, 20);
     a->mincoverage = 0.5;
@@ -83,6 +90,7 @@ static void parse_args(int argc, char **av, cli_args *a) {
         if (strcmp(av[i], "-query") == 0 && nxt) a->query = nxt;
         if (strcmp(av[i], "-db") == 0 && nxt) a->db = nxt;
         if (strcmp(av[i], "-out") == 0 && nxt) a->out = nxt;
+        if (strcmp(av[i], "-out_rev") == 0 && nxt) a->out_rev = nxt;
         if (strcmp(av[i], "-evalue") == 0 && nxt) {
             a->minevalue = (long double)atof(nxt); /* double first, then widened (:553) */
             if (a->minevalue < 0) terror("Min-e-value must be larger than zero");
@@ -118,6 +126,31 @@ static void *ctx_boot_main(void *arg) {
     return NULL;
 }
 
+/* -out_rev: revComp(db) as the loader sees it, built on its own thread while the forward strand is parsed and aligned */
+typedef struct {
+    const char *path;
+    const imsame_fasta *fwd;
+    imsame_fasta rev;
+    int has_u, rc, started, joined;
+    pthread_t thread;
+} rev_load;
+static void *rev_load_main(void *arg) {
+    rev_load *r = (rev_load *)arg;
+    r->rc = imsame_revcomp_load(r->path, &r->rev, &r->has_u);
+    return NULL;
+}
+static const imsame_fasta *rev_wait(void *arg, int *on_device) {
+    rev_load *r = (rev_load *)arg;
+    if (!r->joined) {
+        if (r->started) pthread_join(r->thread, NULL);
+        else rev_load_main(r);
+        r->joined = 1;
+    }
+    if (r->rc) return NULL;
+    if (on_device) *on_device = imsame_revcomp_on_device(r->fwd, &r->rev, r->has_u);
+    return &r->rev;
+}
+
 int main(int argc, char **av) {
     cli_args a;
     parse_args(argc, av, &a);
@@ -127,6 +160,14 @@ int main(int argc, char **av) {
     if (fq == NULL || fd == NULL) terror("A query and database is required");
     fclose(fq);
     fclose(fd);
+    FILE *fout_rev = NULL;
+    rev_load rl;
+    memset(&rl, 0, sizeof rl);
+    if (a.out_rev) {
+        if ((fout_rev = fopen(a.out_rev, "wt")) == NULL) terror("Could not open the reverse-strand output file");
+        rl.path = a.db;
+        rl.started = pthread_create(&rl.thread, NULL, rev_load_main, &rl) == 0;
+    }
 
     double t0 = now_s();
     fprintf(stdout, "[INFO] Init. quick table\n");
@@ -143,6 +184,7 @@ int main(int argc, char **av) {
     t0 = now_s();
     imsame_fasta db, q;
     if (imsame_fasta_load(a.db, 1, &db)) terror("Could not allocate memory for database vector");
+    rl.fwd = &db;
     fprintf(stdout, "[INFO] Database loaded and of length %" PRIu64 ". Hash table building took %e seconds\n",
             db.total_len, now_s() - t0);
     t0 = now_s();
@@ -174,6 +216,14 @@ int main(int argc, char **av) {
     jo.kmer = a.kmer;
     jo.device = a.device;
     jo.trace = getenv("IMSAME_TRACE") != NULL; /* phase wall times on stderr (not part of the reference's output) */
+    imsame_rev_job rj;
+    memset(&rj, 0, sizeof rj);
+    if (a.out_rev) {
+        rj.out = fout_rev;
+        rj.wait = rev_wait;
+        rj.arg = &rl;
+        jo.rev = &rj;
+    }
     char err[300];
     imsame_ctx *ctx = NULL;
     if (booting) {
@@ -197,8 +247,29 @@ int main(int argc, char **av) {
             accepted, q.n_seqs, db.n_seqs, (long double)a.minevalue, (int)(100 * a.mincoverage));
     fprintf(stdout, "[INFO] The Jaccard-index is: %Le\n",
             (long double)accepted / ((db.n_seqs + q.n_seqs) - accepted));
+    if (a.out_rev) {
+        /* what the second process of the workflow (IMSAME -db revComp(db)) would report; revComp writes one record
+           per '>' byte, so its read count is the reverse parse's own */
+        const imsame_fasta *rdb = rev_wait(&rl, NULL);
+        if (rl.rc == 1) terror("opening IN sequence FASTA file");
+        if (rl.rc == 2) terror("memory for Seq");
+        if (rl.rc == 3) terror("Could not allocate memory for database vector");
+        if (rj.rc == IMSAME_EREADSIZE) terror("Read size reached for gapped alignment.");
+        if (rj.rc) {
+            char msg[512];
+            snprintf(msg, sizeof msg, "GPU hot path failed: %s%s%s", imsame_gpu_strerror(rj.rc), err[0] ? " / " : "", err);
+            terror(msg);
+        }
+        fprintf(stdout,
+                "[INFO] %" PRIu64 " reads (%" PRIu64 ") from the query were found in the reverse complement of the database (%" PRIu64
+                ") at a minimum e-value of %Le and minimum coverage of %d%%.\n",
+                rj.accepted, q.n_seqs, rdb->n_seqs, (long double)a.minevalue, (int)(100 * a.mincoverage));
+        fprintf(stdout, "[INFO] The Jaccard-index against the reverse complement is: %Le\n",
+                (long double)rj.accepted / ((rdb->n_seqs + q.n_seqs) - rj.accepted));
+    }
     fprintf(stdout, "[INFO] Deallocating heap memory.\n");
     if (fout != NULL) fclose(fout);
+    if (fout_rev != NULL) fclose(fout_rev);
     fflush(stdout);
     /* Everything the caller can observe is on disk / on stdout now: the process ends here and leaves the device
        memory, the pinned buffers and the parsed reads to the operating system instead of releasing them piece by
@@ -215,6 +286,7 @@ int main(int argc, char **av) {
     t0 = now_s();
     imsame_fasta_free(&db);
     imsame_fasta_free(&q);
+    if (a.out_rev) imsame_fasta_free(&rl.rev);
     if (jo.trace) fprintf(stderr, "[imsame] host read sets freed in %.3f s\n", now_s() - t0);
     return 0;
 }

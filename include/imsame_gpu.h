@@ -196,6 +196,27 @@ int imsame_gpu_align_sharded(imsame_ctx *const *ctxs, int n, const imsame_seqinf
                              const imsame_seqinfo *query, const imsame_params *params, imsame_best *out,
                              imsame_stats *stats);
 
+/* ---- the reverse strand of the resident database --------------------------------------------------
+ * A read may come from either strand; the reference workflow aligns the query once more against revComp(db)
+ * (src/reverseComplement.c) in a second process.  These calls give the records of `IMSAME -db revComp(db)` from
+ * the database already on the device.
+ *
+ * The resident database (set_db, or what the last imsame_gpu_align / _align_shard left resident) becomes its reverse
+ * complement in place: reads in reverse order, each reverse complemented, offsets and word breaks mirrored -- what
+ * revComp + the loader give when imsame_revcomp_is_mirror holds (a break at a segment's first base, which changes
+ * no word, is dropped).  Calling it again restores the forward database.  IMSAME_ESTATE without a resident
+ * database, with a sample's (imsame_gpu_sample_revcomp) or while a run is in progress.
+ * A per-rank caller of a sharded database sets, for the reverse strand, db_pos_base' = T - (db_pos_base + shard bases)
+ * and db_seq_base' = N - (db_seq_base + shard reads) (T, N: bases and reads of the whole database). */
+int imsame_gpu_db_revcomp(imsame_ctx *ctx);
+/* The query, parameters and contexts of the previous imsame_gpu_align (n = 1) / imsame_gpu_align_sharded (same ctxs,
+ * same order) call, aligned against the reverse complement of that call's database, which is still resident: no upload,
+ * no word table rebuilt for the first pass.  out: nq records whose db_seq / db_pos count in the reverse database.
+ * stats: n entries or NULL.  The database stays reversed.  IMSAME_ESTATE when the contexts do not hold the state of
+ * such a call that succeeded; IMSAME_EARG when it had a non-zero db_pos_base / db_seq_base (the whole database is
+ * then unknown); IMSAME_EREADSIZE exactly where the reference stops on revComp(db). */
+int imsame_gpu_align_revcomp(imsame_ctx *const *ctxs, int n, imsame_best *out, imsame_stats *stats);
+
 /* ---- NW on explicit pairs (src/alignmentFunctions.c:389-560 in isolation) */
 /* X[i] / Y[i]: ASCII reads; out5[i*5..] = score, bx, by, length, identities */
 int imsame_gpu_nw_batch(imsame_ctx *ctx, uint32_t n_pairs, const unsigned char *const *X,
