@@ -57,7 +57,7 @@ class Stats(C.Structure):
 
 
 # every symbol declared in include/imsame_gpu.h
-SYMBOLS = ["imsame_gpu_create", "imsame_gpu_destroy", "imsame_gpu_strerror", "imsame_gpu_last_cuda_error",
+SYMBOLS = ["imsame_gpu_create", "imsame_gpu_destroy", "imsame_gpu_strerror", "imsame_gpu_last_cuda_error", "imsame_gpu_mem_info",
            "imsame_gpu_set_stream", "imsame_gpu_align", "imsame_gpu_set_query", "imsame_gpu_set_db",
            "imsame_gpu_run", "imsame_gpu_n_segments", "imsame_gpu_n_bands", "imsame_gpu_run_begin",
            "imsame_gpu_run_scan", "imsame_gpu_run_band", "imsame_gpu_run_select", "imsame_gpu_run_end",
@@ -93,6 +93,7 @@ def lib():
         l.imsame_gpu_strerror.restype = C.c_char_p
         l.imsame_gpu_last_cuda_error.argtypes = [vp]
         l.imsame_gpu_last_cuda_error.restype = C.c_char_p
+        l.imsame_gpu_mem_info.argtypes = [vp, C.POINTER(u64), C.POINTER(u64)]
         l.imsame_gpu_set_stream.argtypes = [vp, vp]
         l.imsame_gpu_align.argtypes = [vp, C.POINTER(SeqInfo), C.POINTER(SeqInfo), C.POINTER(Params), vp,
                                        C.POINTER(Stats)]

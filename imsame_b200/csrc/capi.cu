@@ -136,6 +136,8 @@ struct imsame_ctx {
     int k_tables = 0;
     int q_k = K;      // the seed length the resident query table was built with
     int scan_grid = 0;
+    // test hook IMSAME_TEST_FAIL_ALLOC=N[,M] (read by imsame_gpu_create): device allocations N .. N+M-1 of this context fail
+    uint64_t n_allocs = 0, fail_alloc_first = 0, fail_alloc_count = 0;
 
     // device blocks released by free_query / free_db, reused by the next set_query / set_db
     // (cudaFree + cudaMalloc of the ~3 GB of a cfg2 call cost several hundred ms per call)
@@ -192,17 +194,32 @@ void reset_timing(imsame_ctx *ctx) {
     ctx->launches = ctx->k2_launches = ctx->k3_launches = ctx->k3_packed = 0;
 }
 
+// cudaMalloc of the context.  Under the test hook IMSAME_TEST_FAIL_ALLOC the chosen allocations ask for an impossible
+// size instead: cudaMalloc fails and records the error as on a full device, and no memory outside the process is touched.
+cudaError_t ctx_malloc(imsame_ctx *ctx, void **p, size_t bytes) {
+    const uint64_t i = ++ctx->n_allocs;
+    if (ctx->fail_alloc_first && i >= ctx->fail_alloc_first && i < ctx->fail_alloc_first + ctx->fail_alloc_count) {
+        if (cudaMalloc(p, (size_t)1 << 50) == cudaSuccess) cudaFree(*p);
+        *p = nullptr;
+        return cudaErrorMemoryAllocation;
+    }
+    const cudaError_t e = cudaMalloc(p, bytes);
+    if (e != cudaSuccess) *p = nullptr;
+    return e;
+}
+
 template <typename T>
 int dev_alloc(imsame_ctx *ctx, T **p, uint64_t count) {
     const size_t bytes = (size_t)std::max<uint64_t>(count, 1) * sizeof(T);
-    cudaError_t e = cudaMalloc((void **)p, bytes);
+    cudaError_t e = ctx_malloc(ctx, (void **)p, bytes);
     if (e == cudaErrorMemoryAllocation && !ctx->free_blocks.empty()) {  // give the recycled blocks back and retry
         cudaGetLastError();
         for (auto &b : ctx->free_blocks) cudaFree(b.p);
         ctx->free_blocks.clear();
-        e = cudaMalloc((void **)p, bytes);
+        e = ctx_malloc(ctx, (void **)p, bytes);
     }
     if (e != cudaSuccess) {
+        cudaGetLastError();  // a failed cudaMalloc is not sticky: the next CK(cudaGetLastError()) must not report it again
         ctx->cuda_err = std::string("cudaMalloc: ") + cudaGetErrorString(e);
         return e == cudaErrorMemoryAllocation ? IMSAME_ENOMEM : IMSAME_ECUDA;
     }
@@ -229,14 +246,15 @@ int pool_alloc(imsame_ctx *ctx, T **p, uint64_t count) {
         ctx->free_blocks.erase(ctx->free_blocks.begin() + best);
         return IMSAME_OK;
     }
-    cudaError_t e = cudaMalloc((void **)p, bytes);
+    cudaError_t e = ctx_malloc(ctx, (void **)p, bytes);
     if (e == cudaErrorMemoryAllocation && !ctx->free_blocks.empty()) {  // give the cached blocks back and retry
         cudaGetLastError();
         for (auto &b : ctx->free_blocks) cudaFree(b.p);
         ctx->free_blocks.clear();
-        e = cudaMalloc((void **)p, bytes);
+        e = ctx_malloc(ctx, (void **)p, bytes);
     }
     if (e != cudaSuccess) {
+        cudaGetLastError();  // (as in dev_alloc)
         ctx->cuda_err = std::string("cudaMalloc: ") + cudaGetErrorString(e);
         return e == cudaErrorMemoryAllocation ? IMSAME_ENOMEM : IMSAME_ECUDA;
     }
@@ -393,18 +411,25 @@ int upload_u32(imsame_ctx *ctx, uint32_t *dst, const uint32_t *src, uint64_t n) 
 }
 
 int ensure_work_buffers(imsame_ctx *ctx, uint32_t want_cap) {
-    if (!ctx->d_small) {
+    if (!ctx->d_lut) {  // (the last of them: a call that ran out of memory half way completes the set next time)
         int rc;
-        if ((rc = dev_alloc(ctx, &ctx->d_small, 4))) return rc;
-        if ((rc = dev_alloc(ctx, &ctx->d_counters, 16))) return rc;
-        if ((rc = dev_alloc(ctx, &ctx->d_overflow, 1))) return rc;
-        if ((rc = dev_alloc(ctx, &ctx->d_nmin, EXT_MAX_READ + 1))) return rc;  // every read length the scan admits
-        if ((rc = dev_alloc(ctx, &ctx->d_lmin, IMSAME_MAX_READ_SIZE + 1))) return rc;
-        if ((rc = dev_alloc(ctx, &ctx->d_imin, 2 * IMSAME_MAX_READ_SIZE + 1))) return rc;
-        if ((rc = dev_alloc(ctx, &ctx->d_lut, EXT_LUT3_SIZE))) return rc;
+        if (!ctx->d_small && (rc = dev_alloc(ctx, &ctx->d_small, 4))) return rc;
+        if (!ctx->d_counters && (rc = dev_alloc(ctx, &ctx->d_counters, 16))) return rc;
+        if (!ctx->d_overflow && (rc = dev_alloc(ctx, &ctx->d_overflow, 1))) return rc;
+        if (!ctx->d_nmin && (rc = dev_alloc(ctx, &ctx->d_nmin, EXT_MAX_READ + 1))) return rc;  // every read length the scan admits
+        if (!ctx->d_lmin && (rc = dev_alloc(ctx, &ctx->d_lmin, IMSAME_MAX_READ_SIZE + 1))) return rc;
+        if (!ctx->d_imin && (rc = dev_alloc(ctx, &ctx->d_imin, 2 * IMSAME_MAX_READ_SIZE + 1))) return rc;
+        uint32_t *d_lut = nullptr;
+        if ((rc = dev_alloc(ctx, &d_lut, EXT_LUT3_SIZE))) return rc;
         std::vector<uint32_t> lut(EXT_LUT3_SIZE);
         build_ext_lut3(lut.data());
-        CK(cudaMemcpy(ctx->d_lut, lut.data(), EXT_LUT3_SIZE * sizeof(uint32_t), cudaMemcpyHostToDevice));
+        const cudaError_t e = cudaMemcpy(d_lut, lut.data(), EXT_LUT3_SIZE * sizeof(uint32_t), cudaMemcpyHostToDevice);
+        if (e != cudaSuccess) {
+            cudaFree(d_lut);
+            ctx->cuda_err = std::string("cudaMemcpy: ") + cudaGetErrorString(e);
+            return IMSAME_ECUDA;
+        }
+        ctx->d_lut = d_lut;
     }
     if (want_cap > ctx->hcap) {
         ctx->hcap = 0;  // a failed allocation below must not leave a stale capacity behind
@@ -550,6 +575,7 @@ int ensure_carry(imsame_ctx *ctx, uint32_t max_ylen) {
     const uint64_t warps = (uint64_t)std::max(std::max(ctx->nw_grid[5], ctx->nw_grid[6]), std::max(ctx->nw_grid[7], ctx->nw_grid[8])) * NW_WARPS;
     if (warps > ctx->carry_warps) {
         dev_free(ctx->carry);
+        ctx->carry_warps = 0;  // a failed allocation below must not leave a stale capacity behind
         int rc = dev_alloc(ctx, &ctx->carry, warps * 2 * MAX_READ);
         if (rc) return rc;
         ctx->carry_warps = warps;
@@ -697,6 +723,18 @@ const char *imsame_gpu_strerror(int code) {
 
 const char *imsame_gpu_last_cuda_error(const imsame_ctx *ctx) { return ctx ? ctx->cuda_err.c_str() : ""; }
 
+int imsame_gpu_mem_info(const imsame_ctx *ctx, uint64_t *free_bytes, uint64_t *total_bytes) {
+    if (!ctx || !free_bytes || !total_bytes) return IMSAME_EARG;
+    size_t f = 0, t = 0;
+    if (cudaSetDevice(ctx->device) != cudaSuccess || cudaMemGetInfo(&f, &t) != cudaSuccess) {
+        cudaGetLastError();
+        return IMSAME_ECUDA;
+    }
+    *free_bytes = f;
+    *total_bytes = t;
+    return IMSAME_OK;
+}
+
 int imsame_gpu_create(imsame_ctx **out, int device) {
     if (!out) return IMSAME_EARG;
     *out = nullptr;
@@ -716,6 +754,10 @@ int imsame_gpu_create(imsame_ctx **out, int device) {
     cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, scan_kernel<K>, SCAN_THREADS_K2, 0);
     if (const char *e = getenv("IMSAME_SCAN_BLOCKS_PER_SM")) per_sm = std::min(per_sm, std::max(1, atoi(e)));  // tuning knob
     ctx->scan_grid = std::max(1, per_sm) * ctx->n_sm;
+    if (const char *e = getenv("IMSAME_TEST_FAIL_ALLOC")) {  // test hook: the error paths of running out of device memory
+        unsigned long long first = 0, count = 1;
+        if (sscanf(e, "%llu,%llu", &first, &count) >= 1) { ctx->fail_alloc_first = first; ctx->fail_alloc_count = count; }
+    }
     *out = ctx;
     return IMSAME_OK;
 }
@@ -1010,6 +1052,7 @@ static int run_begin_impl(imsame_ctx *ctx, const imsame_params *p, uint64_t *d_k
     int rc;
     if (ctx->keys_cap < nq) {
         dev_free(ctx->keys); dev_free(ctx->payload); dev_free(ctx->pkey);
+        ctx->keys_cap = 0;  // (as in ensure_work_buffers)
         if ((rc = dev_alloc(ctx, &ctx->keys, nq))) return rc;
         if ((rc = dev_alloc(ctx, &ctx->payload, nq))) return rc;
         if ((rc = dev_alloc(ctx, &ctx->pkey, nq))) return rc;
@@ -1026,6 +1069,7 @@ static int run_begin_impl(imsame_ctx *ctx, const imsame_params *p, uint64_t *d_k
     const uint32_t nseg = (uint32_t)n_lsegs(ctx);
     if (ctx->bins_segs < nseg) {
         dev_free(ctx->d_bins);
+        ctx->bins_segs = 0;
         if ((rc = dev_alloc(ctx, &ctx->d_bins, (uint64_t)nseg * BINS_STRIDE))) return rc;
         ctx->bins_segs = nseg;
     }

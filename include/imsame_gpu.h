@@ -105,6 +105,8 @@ int imsame_gpu_create(imsame_ctx **ctx, int device);
 void imsame_gpu_destroy(imsame_ctx *ctx);
 const char *imsame_gpu_strerror(int code);
 const char *imsame_gpu_last_cuda_error(const imsame_ctx *ctx);
+/* free and total memory of the context's device (cudaMemGetInfo) */
+int imsame_gpu_mem_info(const imsame_ctx *ctx, uint64_t *free_bytes, uint64_t *total_bytes);
 /* run all work of this context on an existing cudaStream_t (NULL = own non-blocking stream; pass
  * cudaStreamLegacy / cudaStreamPerThread to share a default stream with other libraries) */
 int imsame_gpu_set_stream(imsame_ctx *ctx, void *cuda_stream);
@@ -263,7 +265,11 @@ int imsame_gpu_set_kmer(imsame_ctx *ctx, int k);
  * a record is a word break of the sample but not of its reverse complement, and revComp turns U into
  * an A the loader keeps.  imsame_revcomp_is_mirror (imsame_b200/host/imsame_host.h) decides it on the
  * two parses; otherwise upload the parse of revComp's text with imsame_gpu_sample_create.
- * A sample used as a database must fit one segment (2^29 bases, IMSAME_ELIMIT otherwise). */
+ * A sample used as a database must fit one segment (2^29 bases, IMSAME_ELIMIT otherwise).
+ * A sample belongs to the context it was made with: imsame_gpu_align_samples points the context at the
+ * query's buffers and stores the word table in the query sample, so two contexts never share one.
+ * After any error of imsame_gpu_align_samples (IMSAME_ENOMEM included) the context and both samples stay
+ * usable: free memory and call it again, or fall back to imsame_gpu_align. */
 typedef struct imsame_sample imsame_sample;
 int imsame_gpu_sample_create(imsame_ctx *ctx, const imsame_seqinfo *reads, imsame_sample **out);
 int imsame_gpu_sample_revcomp(imsame_ctx *ctx, const imsame_sample *in, imsame_sample **out);
