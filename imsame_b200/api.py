@@ -17,6 +17,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 GPU_SO = os.environ.get("IMSAME_GPU_SO") or os.path.join(_HERE, "_lib", "libimsame_gpu.so")  # override: experiments
 
 KEY_NONE = 0x7FFFFFFFFFFFFFFF
+SWEEP_MAX = 16  # IMSAME_SWEEP_MAX
 
 
 class SeqInfo(C.Structure):
@@ -64,7 +65,7 @@ SYMBOLS = ["imsame_gpu_create", "imsame_gpu_destroy", "imsame_gpu_strerror", "im
            "imsame_gpu_mask_payload", "imsame_gpu_fetch", "imsame_gpu_nw_batch", "imsame_gpu_set_nw_mode", "imsame_gpu_set_passes",
            "imsame_gpu_set_kmer", "imsame_gpu_comm_id", "imsame_gpu_comm_init", "imsame_gpu_comm_free",
            "imsame_gpu_run_sharded", "imsame_gpu_align_shard", "imsame_gpu_align_sharded",
-           "imsame_gpu_db_revcomp", "imsame_gpu_align_revcomp",
+           "imsame_gpu_db_revcomp", "imsame_gpu_align_revcomp", "imsame_gpu_align_sweep",
            "imsame_gpu_sample_create", "imsame_gpu_sample_revcomp", "imsame_gpu_sample_free", "imsame_gpu_align_samples",
            "imsame_gpu_traceback", "imsame_gpu_free", "imsame_gpu_host_alloc", "imsame_gpu_host_free"]
 
@@ -97,6 +98,8 @@ def lib():
         l.imsame_gpu_set_stream.argtypes = [vp, vp]
         l.imsame_gpu_align.argtypes = [vp, C.POINTER(SeqInfo), C.POINTER(SeqInfo), C.POINTER(Params), vp,
                                        C.POINTER(Stats)]
+        l.imsame_gpu_align_sweep.argtypes = [vp, C.POINTER(SeqInfo), C.POINTER(SeqInfo), vp, C.c_int, vp, vp,
+                                             C.POINTER(Stats)]
         l.imsame_gpu_set_query.argtypes = [vp, C.POINTER(SeqInfo), C.POINTER(Params)]
         l.imsame_gpu_set_db.argtypes = [vp, C.POINTER(SeqInfo)]
         l.imsame_gpu_run.argtypes = [vp, C.POINTER(Params), vp, vp, C.POINTER(Stats)]
@@ -260,6 +263,23 @@ class Imsame:
                                            C.byref(st)))
         self.nq = int(q.n_seqs)
         return out, st.as_dict()
+
+    def align_sweep(self, db, query, params_list, db_breaks=None):
+        """one run, several coverage/identity sets (imsame_gpu_align_sweep): params_list = Params that differ only in
+        min_coverage / min_identity (at most SWEEP_MAX).  Returns ([records per set], [IMSAME_OK or IMSAME_EREADSIZE
+        per set], stats): set t's records are what align() with params_list[t] returns; a set whose code is not 0
+        has all-zero records."""
+        d, k1 = _seqinfo(db[0], db[1], db_breaks)
+        q, k2 = _seqinfo(query[0], query[1])
+        n, nq = len(params_list), int(q.n_seqs)
+        ps = (Params * max(n, 1))(*params_list)
+        out = np.zeros(max(n, 1) * nq, dtype=BEST_DTYPE)
+        codes = np.zeros(max(n, 1), dtype=np.int32)
+        st = Stats()
+        self._check(lib().imsame_gpu_align_sweep(self._h, C.byref(d), C.byref(q), C.cast(ps, C.c_void_p), n,
+                                                 out.ctypes.data, codes.ctypes.data, C.byref(st)))
+        self.nq = nq
+        return [out[t * nq:(t + 1) * nq].copy() for t in range(n)], [int(c) for c in codes[:n]], st.as_dict()
 
     # -- staged form
     def set_query(self, query, params=None):

@@ -19,6 +19,7 @@
 #include "qtable.cuh"
 #include "revcomp.cuh"
 #include "scan.cuh"
+#include "sweep.cuh"
 
 using namespace imsame;
 
@@ -107,6 +108,11 @@ struct imsame_ctx {
     imsame_params run_params;
     bool run_active = false;
     bool run_masked = false;   // the payloads of superseded keys have been dropped (run_mask)
+    // threshold sweep (capi_sweep.inc): per-set keys and payloads (sweep_cap = sets x reads they hold), the
+    // per-set filter tables (SWEEP_MAX of each) and read-size flags
+    unsigned long long *sw_best = nullptr, *sw_payload = nullptr, *sw_flags = nullptr;
+    uint64_t sweep_cap = 0;
+    uint16_t *sw_lmin = nullptr, *sw_imin = nullptr;
     // communicator of a sharded database (capi_sharded.inc): NCCL over NVLink, one rank per GPU
     void *comm = nullptr;
     int comm_rank = 0, comm_size = 1;
@@ -774,6 +780,7 @@ void imsame_gpu_destroy(imsame_ctx *ctx) {
     dev_free(ctx->hkeys); dev_free(ctx->hvals); dev_free(ctx->pairs); dev_free(ctx->res);
     dev_free(ctx->d_small); dev_free(ctx->d_counters); dev_free(ctx->d_overflow);
     dev_free(ctx->keys); dev_free(ctx->payload); dev_free(ctx->pkey); dev_free(ctx->d_bins); dev_free(ctx->carry); dev_free(ctx->stage);
+    dev_free(ctx->sw_best); dev_free(ctx->sw_payload); dev_free(ctx->sw_flags); dev_free(ctx->sw_lmin); dev_free(ctx->sw_imin);
     if (ctx->tb_pin) cudaFreeHost(ctx->tb_pin);
     for (int b = 0; b < 2; b++) {
         if (ctx->pin[b]) cudaFreeHost(ctx->pin[b]);
@@ -1808,3 +1815,4 @@ int imsame_gpu_traceback(imsame_ctx *ctx, const imsame_seqinfo *db, const imsame
 
 #include "capi_sharded.inc"
 #include "capi_samples.inc"
+#include "capi_sweep.inc"

@@ -59,6 +59,12 @@ void imsame_build_lmin(long double min_coverage, uint16_t *lmin);
 /* imin[len], len in [0, 2*IMSAME_MAX_READ_SIZE]: smallest identities with
  * (long double)identities/len >= min_identity; 65535 = never. imin[0] = 65535 (NaN rejects). */
 void imsame_build_imin(long double min_identity, uint16_t *imin);
+/* the tables of n_sets coverage/identity pairs (imsame_gpu_align_sweep): lmin_sets / imin_sets hold n_sets
+ * consecutive tables of IMSAME_MAX_READ_SIZE + 1 / 2 * IMSAME_MAX_READ_SIZE + 1 entries (imsame_build_lmin /
+ * imsame_build_imin of each set); lmin_all / imin_all their elementwise maxima: a pair passes every set exactly
+ * when it passes those. */
+void imsame_build_sweep_tables(int n_sets, const long double *coverage, const long double *identity, uint16_t *lmin_sets,
+                               uint16_t *imin_sets, uint16_t *lmin_all, uint16_t *imin_all);
 
 /* ---- output ---------------------------------------------------------------- */
 /* header line of a record, src/alignmentFunctions.c:167 */

@@ -30,22 +30,47 @@ static void *ctx_main(void *arg) {
     return NULL;
 }
 
-/* traceback on the GPU + rendering of the records of the accepted reads of `best` (db: what best[].db_seq indexes) */
-static int write_records(imsame_ctx **ctx, const imsame_job_opts *o, const imsame_fasta *qf, const imsame_fasta *dbf,
-                         const imsame_params *p, const imsame_best *best, FILE *fout, char *err, size_t errlen, double *tp) {
-    const imsame_fasta q = *qf, db = *dbf;
+/* one traceback on the GPU: the ops and cells of the accepted reads of a record array */
+typedef struct {
+    uint64_t *ops_off;
+    uint32_t *ops, *cell;
+} tb_layer;
+
+static void tb_layer_free(tb_layer *L) {
+    imsame_gpu_free(L->ops);
+    free(L->ops_off);
+    free(L->cell);
+    memset(L, 0, sizeof *L);
+}
+
+static int tb_layer_run(imsame_ctx **ctx, const imsame_job_opts *o, const imsame_fasta *q, const imsame_fasta *db,
+                        const imsame_params *p, const imsame_best *best, tb_layer *L, char *err, size_t errlen, double *tp) {
     imsame_seqinfo qv, dv;
-    imsame_fasta_view(&q, &qv);
-    imsame_fasta_view(&db, &dv);
+    imsame_fasta_view(q, &qv);
+    imsame_fasta_view(db, &dv);
+    memset(L, 0, sizeof *L);
     int rc = IMSAME_OK;
     if (!*ctx && (rc = imsame_gpu_create(ctx, o->device))) return rc;
-    uint64_t *ops_off = (uint64_t *)malloc((q.n_seqs + 1) * sizeof(uint64_t));
-    uint32_t *cell = (uint32_t *)malloc(4 * q.n_seqs * sizeof(uint32_t)), *ops = NULL;
-    rc = (ops_off && cell) ? imsame_gpu_traceback(*ctx, &dv, &qv, p, best, ops_off, &ops, cell) : IMSAME_ENOMEM;
+    L->ops_off = (uint64_t *)malloc((q->n_seqs + 1) * sizeof(uint64_t));
+    L->cell = (uint32_t *)malloc(4 * q->n_seqs * sizeof(uint32_t));
+    rc = (L->ops_off && L->cell) ? imsame_gpu_traceback(*ctx, &dv, &qv, p, best, L->ops_off, &L->ops, L->cell) : IMSAME_ENOMEM;
     if (rc) {
         if (err && errlen) snprintf(err, errlen, "%s", imsame_gpu_last_cuda_error(*ctx));
-    } else {
-        if (o->trace) { fprintf(stderr, "[imsame] traceback (GPU) %.3f s\n", now_s() - *tp); *tp = now_s(); }
+        tb_layer_free(L);
+    } else if (o->trace) {
+        fprintf(stderr, "[imsame] traceback (GPU) %.3f s\n", now_s() - *tp);
+        *tp = now_s();
+    }
+    return rc;
+}
+
+/* rendering of the records of the accepted reads of `best` (db: what best[].db_seq indexes); the path of read r is in
+   layers[layer_of ? layer_of[r] : 0] */
+static int render_records(const imsame_job_opts *o, const imsame_fasta *qf, const imsame_fasta *dbf, const imsame_best *best,
+                          const tb_layer *layers, const uint8_t *layer_of, FILE *fout, double *tp) {
+    const imsame_fasta q = *qf, db = *dbf;
+    int rc = IMSAME_OK;
+    {
         /* records are rendered by all host threads, each into its own buffer for a contiguous range of
            reads, and written in ascending read order (the reference's order with -n_threads 1) */
         int nt = 1;
@@ -73,13 +98,14 @@ static int write_records(imsame_ctx **ctx, const imsame_job_opts *o, const imsam
                     if (!nb2) { free(buf); buf = NULL; break; }
                     buf = nb2;
                 }
+                const tb_layer *L = layers + (layer_of ? layer_of[r] : 0);
                 const uint64_t s = best[r].db_seq;
                 const uint32_t xlen = (uint32_t)(db.start_pos[s + 1] - db.start_pos[s]);
                 const uint32_t ylen = (uint32_t)(q.start_pos[r + 1] - q.start_pos[r]);
                 len += (size_t)imsame_format_header(buf + len, r, s, best[r].length, best[r].identities, ylen);
                 len += (size_t)imsame_render_alignment(buf + len, db.sequences + db.start_pos[s], xlen,
-                                                       q.sequences + q.start_pos[r], ylen, cell[4 * r], cell[4 * r + 1],
-                                                       ops + ops_off[r], ops_off[r + 1] - ops_off[r]);
+                                                       q.sequences + q.start_pos[r], ylen, L->cell[4 * r], L->cell[4 * r + 1],
+                                                       L->ops + L->ops_off[r], L->ops_off[r + 1] - L->ops_off[r]);
             }
             if (!buf) {
 #pragma omp atomic write
@@ -95,9 +121,106 @@ static int write_records(imsame_ctx **ctx, const imsame_job_opts *o, const imsam
         if (failed) rc = IMSAME_ENOMEM;
         if (o->trace) { fprintf(stderr, "[imsame] render + write %.3f s\n", now_s() - *tp); *tp = now_s(); }
     }
-    imsame_gpu_free(ops);
-    free(ops_off);
-    free(cell);
+    return rc;
+}
+
+/* traceback on the GPU + rendering of the records of the accepted reads of `best` */
+static int write_records(imsame_ctx **ctx, const imsame_job_opts *o, const imsame_fasta *q, const imsame_fasta *db,
+                         const imsame_params *p, const imsame_best *best, FILE *fout, char *err, size_t errlen, double *tp) {
+    tb_layer L;
+    int rc = tb_layer_run(ctx, o, q, db, p, best, &L, err, errlen, tp);
+    if (rc) return rc;
+    rc = render_records(o, q, db, best, &L, NULL, fout, tp);
+    tb_layer_free(&L);
+    return rc;
+}
+
+/* the records of n_sets record arrays (best + t * nq) into fouts[t] (NULL: none).  Most sets share most winners: each
+   distinct (read, db_seq) winner is traced once.  Layer L holds the L-th distinct winner of every read (in set order),
+   so that at most n_sets tracebacks together trace every distinct pair exactly once. */
+static int write_sweep_records(imsame_ctx **ctx, const imsame_job_opts *o, const imsame_fasta *q, const imsame_fasta *db,
+                               const imsame_params *p, const imsame_best *best, int n_sets, FILE *const *fouts, char *err,
+                               size_t errlen, double *tp) {
+    const uint64_t nq = q->n_seqs;
+    uint8_t *layer_of = (uint8_t *)calloc((size_t)n_sets * nq, 1);
+    imsame_best *lb = (imsame_best *)malloc(nq * sizeof(imsame_best));
+    if (!layer_of || !lb) { free(layer_of); free(lb); return IMSAME_ENOMEM; }
+    int n_layers = 0;
+    for (uint64_t r = 0; r < nq; r++) {
+        uint64_t seen[IMSAME_SWEEP_MAX];
+        int k = 0;
+        for (int t = 0; t < n_sets; t++) {
+            const imsame_best *b = best + (uint64_t)t * nq + r;
+            if (!fouts[t] || !b->accepted) continue;
+            int j = 0;
+            while (j < k && seen[j] != b->db_seq) j++;
+            if (j == k) seen[k++] = b->db_seq;
+            layer_of[(uint64_t)t * nq + r] = (uint8_t)j;
+        }
+        if (k > n_layers) n_layers = k;
+    }
+    tb_layer layers[IMSAME_SWEEP_MAX];
+    memset(layers, 0, sizeof layers);
+    int rc = IMSAME_OK;
+    for (int L = 0; L < n_layers && !rc; L++) {
+        memset(lb, 0, nq * sizeof(imsame_best));
+        for (uint64_t r = 0; r < nq; r++)
+            for (int t = 0; t < n_sets && !lb[r].accepted; t++) {
+                const imsame_best *b = best + (uint64_t)t * nq + r;
+                if (fouts[t] && b->accepted && layer_of[(uint64_t)t * nq + r] == L) lb[r] = *b;
+            }
+        rc = tb_layer_run(ctx, o, q, db, p, lb, &layers[L], err, errlen, tp);
+    }
+    for (int t = 0; t < n_sets && !rc; t++)
+        if (fouts[t]) rc = render_records(o, q, db, best + (uint64_t)t * nq, layers, layer_of + (uint64_t)t * nq, fouts[t], tp);
+    for (int L = 0; L < n_layers; L++) tb_layer_free(&layers[L]);
+    free(layer_of);
+    free(lb);
+    return rc;
+}
+
+/* o->sweep: the job's thresholds as set 0 of imsame_gpu_align_sweep, the sweep's entries as sets 1 .. n */
+static int sweep_job(const imsame_fasta *q, const imsame_fasta *db, const imsame_job_opts *o, const imsame_params *p,
+                     int kmer, FILE *fout, imsame_ctx **ctx_cache, uint64_t *accepted_out, char *err, size_t errlen) {
+    imsame_sweep_job *sw = o->sweep;
+    const int n_sets = 1 + sw->n;
+    if (n_sets > IMSAME_SWEEP_MAX || o->gpus > 1 || o->rev || o->q_sample) return IMSAME_EARG;
+    double tp = now_s();
+    imsame_seqinfo qv, dv;
+    imsame_fasta_view(q, &qv);
+    imsame_fasta_view(db, &dv);
+    imsame_params ps[IMSAME_SWEEP_MAX];
+    for (int t = 0; t < n_sets; t++) {
+        ps[t] = *p;
+        if (t) { ps[t].min_coverage = sw->coverage[t - 1]; ps[t].min_identity = sw->identity[t - 1]; }
+    }
+    const uint64_t nq = q->n_seqs;
+    imsame_best *best = (imsame_best *)calloc((size_t)n_sets * nq, sizeof(imsame_best));
+    if (!best) return IMSAME_ENOMEM;
+    int set_rc[IMSAME_SWEEP_MAX];
+    imsame_ctx *ctx = (ctx_cache && *ctx_cache) ? *ctx_cache : NULL;
+    int rc = IMSAME_OK;
+    if (!ctx && (rc = imsame_gpu_create(&ctx, o->device))) { free(best); return rc; }
+    if (ctx_cache) *ctx_cache = ctx;
+    rc = imsame_gpu_set_kmer(ctx, kmer);
+    if (!rc) rc = imsame_gpu_align_sweep(ctx, &dv, &qv, ps, n_sets, best, set_rc, NULL);
+    if (rc && err && errlen) snprintf(err, errlen, "%s", imsame_gpu_last_cuda_error(ctx));
+    if (!rc) rc = set_rc[0];  /* the main set's read-size stop ends the job as without the sweep */
+    if (!rc) {
+        if (o->trace) { fprintf(stderr, "[imsame] align (%d threshold sets) %.3f s\n", n_sets, now_s() - tp); tp = now_s(); }
+        FILE *fouts[IMSAME_SWEEP_MAX];
+        for (int t = 0; t < n_sets; t++) {
+            uint64_t acc = 0;
+            for (uint64_t r = 0; r < nq; r++) acc += best[(uint64_t)t * nq + r].accepted;
+            if (t) { sw->accepted[t - 1] = acc; sw->rc[t - 1] = set_rc[t]; }
+            else *accepted_out = acc;
+            fouts[t] = t ? (sw->out ? sw->out[t - 1] : NULL) : fout;
+            if (set_rc[t] || acc == 0) fouts[t] = NULL;
+        }
+        rc = write_sweep_records(&ctx, o, q, db, p, best, n_sets, fouts, err, errlen, &tp);
+    }
+    if (ctx && !(ctx_cache && *ctx_cache == ctx)) imsame_gpu_destroy(ctx);
+    free(best);
     return rc;
 }
 
@@ -158,6 +281,10 @@ int imsame_run_job(const imsame_fasta *qf, const imsame_fasta *dbf, const imsame
     p.egap = o->egap;
     p.n_threads = o->n_threads;
     const int kmer = o->kmer ? o->kmer : 12; /* FIXED_K, src/structs.h:15 */
+    if (o->sweep) {
+        free(best);
+        return sweep_job(&q, &db, o, &p, kmer, fout, ctx_cache, accepted_out, err, errlen);
+    }
 
     int ng = o->gpus < 1 ? 1 : o->gpus;
     if ((uint64_t)ng > db.n_seqs) ng = (int)db.n_seqs;

@@ -22,6 +22,16 @@ typedef struct imsame_rev_job {
     int rc;            /* out: the reverse strand's result (the job returns the forward strand's) */
 } imsame_rev_job;
 
+/* More coverage/identity sets in the same run (IMSAME -sweep): sets 1 .. n of imsame_gpu_align_sweep, the job's own
+ * thresholds being set 0, whose records and count the job reports as without a sweep.  One GPU, no samples, no rev. */
+typedef struct imsame_sweep_job {
+    int n;
+    const long double *coverage, *identity; /* n each */
+    FILE **out;                             /* n files for the records (NULL, or NULL entries: count only) */
+    uint64_t *accepted;                     /* out: n */
+    int *rc;                                /* out: n, IMSAME_OK or IMSAME_EREADSIZE */
+} imsame_sweep_job;
+
 typedef struct imsame_job_opts {
     uint64_t n_threads;
     long double minevalue, mincoverage, minidentity;
@@ -35,6 +45,8 @@ typedef struct imsame_job_opts {
     const imsame_sample *db_sample;
     /* optional (not with the samples): the reverse strand too, after the forward records are written */
     imsame_rev_job *rev;
+    /* optional (gpus == 1, not with the samples or rev): more threshold sets in the same run */
+    imsame_sweep_job *sweep;
 } imsame_job_opts;
 
 /* Aligns every read of q against db and writes the records of the accepted reads to fout (may be

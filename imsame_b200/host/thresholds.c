@@ -71,3 +71,17 @@ void imsame_build_imin(long double min_identity, uint16_t *imin) {
         imin[len] = (uint16_t)lo;
     }
 }
+
+void imsame_build_sweep_tables(int n_sets, const long double *coverage, const long double *identity, uint16_t *lmin_sets,
+                               uint16_t *imin_sets, uint16_t *lmin_all, uint16_t *imin_all) {
+    const uint64_t nl = IMSAME_MAX_READ_SIZE + 1, ni = 2 * IMSAME_MAX_READ_SIZE + 1;
+    for (uint64_t i = 0; i < nl; i++) lmin_all[i] = 0;
+    for (uint64_t i = 0; i < ni; i++) imin_all[i] = 0;
+    for (int t = 0; t < n_sets; t++) {
+        uint16_t *l = lmin_sets + (uint64_t)t * nl, *m = imin_sets + (uint64_t)t * ni;
+        imsame_build_lmin(coverage[t], l);
+        imsame_build_imin(identity[t], m);
+        for (uint64_t i = 0; i < nl; i++) if (l[i] > lmin_all[i]) lmin_all[i] = l[i];
+        for (uint64_t i = 0; i < ni; i++) if (m[i] > imin_all[i]) imin_all[i] = m[i];
+    }
+}

@@ -145,3 +145,21 @@ def threshold_tables(min_e_value, min_coverage, min_identity, db_total_len, max_
     lib().imsame_build_lmin(C.c_longdouble(min_coverage), lmin.ctypes.data_as(u16p))
     lib().imsame_build_imin(C.c_longdouble(min_identity), imin.ctypes.data_as(u16p))
     return nmin, lmin, imin
+
+
+def sweep_tables(coverages, identities, max_read=3000):
+    """imsame_build_sweep_tables: (lmin_sets [n, max_read + 1], imin_sets [n, 2 max_read + 1], lmin_all, imin_all);
+    the thresholds pass through double before widening, like make_params"""
+    n = len(coverages)
+    cov = np.array([float(c) for c in coverages], dtype=np.longdouble)
+    idn = np.array([float(i) for i in identities], dtype=np.longdouble)
+    lmin_sets = np.zeros((n, max_read + 1), dtype=np.uint16)
+    imin_sets = np.zeros((n, 2 * max_read + 1), dtype=np.uint16)
+    lmin_all = np.zeros(max_read + 1, dtype=np.uint16)
+    imin_all = np.zeros(2 * max_read + 1, dtype=np.uint16)
+    l = lib()
+    l.imsame_build_sweep_tables.argtypes = [C.c_int] + [C.c_void_p] * 6
+    l.imsame_build_sweep_tables.restype = None
+    l.imsame_build_sweep_tables(n, cov.ctypes.data, idn.ctypes.data, lmin_sets.ctypes.data, imin_sets.ctypes.data,
+                                lmin_all.ctypes.data, imin_all.ctypes.data)
+    return lmin_sets, imin_sets, lmin_all, imin_all

@@ -219,6 +219,29 @@ int imsame_gpu_db_revcomp(imsame_ctx *ctx);
  * then unknown); IMSAME_EREADSIZE exactly where the reference stops on revComp(db). */
 int imsame_gpu_align_revcomp(imsame_ctx *const *ctxs, int n, imsame_best *out, imsame_stats *stats);
 
+/* ---- several coverage / identity threshold sets in one run ------------------------------------------
+ * Metagenomes are compared at more than one similarity level; the reference workflow runs one IMSAME process per
+ * threshold.  Only the filter of the NW epilogue (src/alignmentFunctions.c:163) and the first-accepted selection
+ * after it depend on -coverage / -identity: word table, seed hits, e-value test, candidate pairs and the NW result of
+ * every pair are the same for every set, so one run gives the records of n_sets threshold sets.
+ *   params[0 .. n_sets): full parameter sets that agree exactly in every field but min_coverage and min_identity
+ *                        (e-value, gaps, n_threads, db_*); otherwise IMSAME_EARG.  1 <= n_sets <= IMSAME_SWEEP_MAX.
+ *   out:                 n_sets x nq records; block t (out + t * nq) equals, field by field, what imsame_gpu_align
+ *                        with params[t] returns.
+ *   set_rc[t]:           IMSAME_OK, or IMSAME_EREADSIZE exactly where a separate imsame_gpu_align of set t stops with
+ *                        "Read size reached for gapped alignment." (a candidate with a read of more than
+ *                        IMSAME_MAX_READ_SIZE bases earlier in scan order than set t's final key); that set's block is
+ *                        zeroed, the others are complete.  The call returns 0 when the run completed.
+ *   stats:               one for the run (its n_accepted is set 0's), or NULL.
+ * imsame_gpu_set_kmer / _set_passes / _set_nw_mode apply as to imsame_gpu_align; the context stays usable after
+ * every error.  Device memory: 16 bytes per set and query read on top of imsame_gpu_align.  Not covered: databases
+ * sharded over several GPUs, resident samples (imsame_gpu_align_samples), imsame_gpu_align_revcomp after a sweep
+ * (IMSAME_ESTATE), and sweeping the e-value, the gaps or the seed length. */
+#define IMSAME_SWEEP_MAX 16
+int imsame_gpu_align_sweep(imsame_ctx *ctx, const imsame_seqinfo *db, const imsame_seqinfo *query,
+                           const imsame_params *params, int n_sets, imsame_best *out, int *set_rc,
+                           imsame_stats *stats);
+
 /* ---- NW on explicit pairs (src/alignmentFunctions.c:389-560 in isolation) */
 /* X[i] / Y[i]: ASCII reads; out5[i*5..] = score, bx, by, length, identities */
 int imsame_gpu_nw_batch(imsame_ctx *ctx, uint32_t n_pairs, const unsigned char *const *X,
