@@ -67,6 +67,7 @@ SYMBOLS = ["imsame_gpu_create", "imsame_gpu_destroy", "imsame_gpu_strerror", "im
            "imsame_gpu_run_sharded", "imsame_gpu_align_shard", "imsame_gpu_align_sharded",
            "imsame_gpu_db_revcomp", "imsame_gpu_align_revcomp", "imsame_gpu_align_sweep",
            "imsame_gpu_sample_create", "imsame_gpu_sample_revcomp", "imsame_gpu_sample_free", "imsame_gpu_align_samples",
+           "imsame_gpu_align_samples_sweep",
            "imsame_gpu_traceback", "imsame_gpu_free", "imsame_gpu_host_alloc", "imsame_gpu_host_free"]
 
 _lib = None
@@ -132,6 +133,7 @@ def lib():
         l.imsame_gpu_sample_free.argtypes = [vp, vp]
         l.imsame_gpu_sample_free.restype = None
         l.imsame_gpu_align_samples.argtypes = [vp, vp, vp, C.POINTER(Params), vp, C.POINTER(Stats)]
+        l.imsame_gpu_align_samples_sweep.argtypes = [vp, vp, vp, vp, C.c_int, vp, vp, C.POINTER(Stats)]
         l.imsame_gpu_free.argtypes = [vp]
         l.imsame_gpu_free.restype = None
         l.imsame_gpu_host_alloc.argtypes = [u64]
@@ -352,6 +354,20 @@ class Imsame:
         self._check(lib().imsame_gpu_align_samples(self._h, db._h, query._h, C.byref(params), out.ctypes.data, C.byref(st)))
         self.nq = query.n
         return out, st.as_dict()
+
+    def align_samples_sweep(self, db, query, params_list):
+        """align_sweep with both read sets resident (imsame_gpu_align_samples_sweep): returns ([records per set],
+        [IMSAME_OK or IMSAME_EREADSIZE per set], stats); set t's records are what align_samples() with params_list[t]
+        returns"""
+        n, nq = len(params_list), query.n
+        ps = (Params * max(n, 1))(*params_list)
+        out = np.zeros(max(n, 1) * nq, dtype=BEST_DTYPE)
+        codes = np.zeros(max(n, 1), dtype=np.int32)
+        st = Stats()
+        self._check(lib().imsame_gpu_align_samples_sweep(self._h, db._h, query._h, C.cast(ps, C.c_void_p), n,
+                                                         out.ctypes.data, codes.ctypes.data, C.byref(st)))
+        self.nq = nq
+        return [out[t * nq:(t + 1) * nq].copy() for t in range(n)], [int(c) for c in codes[:n]], st.as_dict()
 
     # -- database sharded over several GPUs, reduced by NCCL inside the library
     def comm_init(self, comm_id, n_ranks, rank):

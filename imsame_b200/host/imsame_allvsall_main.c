@@ -11,12 +11,23 @@
  * processes for 8 samples and re-parses every file 14 times.
  *
  * usage: IMSAME_allvsall metagenomes_directory coverage similarity threads file_extension outpath
- *                        [-device D] [-gpus N] [-jobs J]
+ *                        [-device D] [-gpus N] [-jobs J] [-sweep C1:I1[,C2:I2...]]
  *   -device D   first CUDA device (default 0)
  *   -gpus N     use the devices D .. D+N-1 (default 1)
  *   -jobs J     comparisons in flight (default N): J worker threads, each with its own CUDA context, go
  *               round-robin over the N devices.  J > N puts several workers on one GPU, so that one
  *               renders its records while another aligns.  The output files do not depend on N or J.
+ *   -sweep L    up to 15 more coverage:identity pairs (grammar, limit and errors of IMSAME -sweep), evaluated in the
+ *               same alignment of every unit (imsame_gpu_align_samples_sweep; imsame_gpu_align_sweep for a unit that
+ *               runs from host buffers).  Entry i's records go to OUT/X-Y.align.i and OUT/X-Y.r.align.i (i from 1),
+ *               byte-identical to the X-Y.align / X-Y.r.align of a separate run with coverage Ci and similarity Ii;
+ *               X-Y.align stays what the run without -sweep writes.  After each unit's [INFO] line comes one line per
+ *               entry, "[INFO] X vs Y[ (reverse complement)] sweep i of n (-coverage Ci -identity Ii): A reads (nq)
+ *               from the query were found in the database (ndb); Jaccard-index J", values as given.  A read-size stop
+ *               of entry i (where a separate run at that threshold would have stopped the whole run) writes no .i file
+ *               for that unit and prints the reference's "ERR**** Read size reached for gapped alignment. ****" in
+ *               place of the entry's line; the run goes on and ends with exit status 255.  A stop of the main
+ *               thresholds fails the unit as without -sweep.
  *
  * A unit is one output file (X, Y, strand); the canonical order is the script's loop order.  A free worker
  * takes the next pending unit, preferring one whose query sample's word table it holds, then one whose
@@ -32,7 +43,10 @@
  * running unit needs any more is released; to make room, the least recently used read sets that the unit
  * does not need are evicted.  A unit whose read sets do not fit the budget on their own, whose database is
  * larger than one segment (2^29 bases), or that still meets IMSAME_ENOMEM after everything else was
- * evicted, runs from host buffers (imsame_gpu_align).
+ * evicted, runs from host buffers (imsame_gpu_align).  With -sweep, a unit's per-set key arrays (16 bytes per set and
+ * query read) come out of the half of free memory left for work buffers; the IMSAME_ENOMEM retry and the host-buffer
+ * fallback cover them too.  Resume rule with -sweep: a unit is skipped when its main file and all n entry files
+ * exist; otherwise all of them are written again.
  *
  * Environment: IMSAME_TRACE (phase times; one line per worker at the end: device, units, uploads, table
  * builds, evictions, host-path fallbacks, busy seconds), IMSAME_NO_RESIDENT (every unit from host buffers),
@@ -116,6 +130,8 @@ static struct {
     imsame_job_opts jo;
     int no_resident, n_gpus, n_workers, omp_threads;
     long long test_budget; /* IMSAME_TEST_SAMPLE_BUDGET, -1 = none */
+    imsame_sweep_list sw;  /* -sweep */
+    int entry_stops;       /* -sweep entries that stopped on the read size (G.lock) */
 } G;
 
 static int by_name(const void *a, const void *b) { return strcoll(((const sample *)a)->name, ((const sample *)b)->name); }
@@ -127,6 +143,33 @@ static int exists(const char *path) {
 
 static void unit_path(const unit *u, char *path, size_t len) {
     snprintf(path, len, "%s/%s-%s%s.align", G.out, G.sm[u->i].name, G.sm[u->j].name, u->rev ? ".r" : "");
+}
+
+/* -sweep entry i (from 1) of a unit: its main file's path + ".i" */
+static void entry_path(const unit *u, int i, char *path, size_t len) {
+    snprintf(path, len, "%s/%s-%s%s.align.%d", G.out, G.sm[u->i].name, G.sm[u->j].name, u->rev ? ".r" : "", i);
+}
+
+/* resume rule: the main file and every entry file exist */
+static int unit_done(const unit *u) {
+    char path[4096];
+    unit_path(u, path, sizeof path);
+    if (!exists(path)) return 0;
+    for (int i = 1; i <= G.sw.n; i++) {
+        entry_path(u, i, path, sizeof path);
+        if (!exists(path)) return 0;
+    }
+    return 1;
+}
+
+/* (re)opens the entry files of a unit for writing */
+static void open_entries(const unit *u, FILE **f) {
+    for (int i = 0; i < G.sw.n; i++) {
+        char path[4096];
+        entry_path(u, i + 1, path, sizeof path);
+        if (f[i]) fclose(f[i]);
+        f[i] = fopen(path, "wt");
+    }
 }
 
 /* ---- host parses (shared, read-only once built) ---- */
@@ -306,6 +349,20 @@ static int run_unit(worker *w, unit *u) {
     char path[4096];
     unit_path(u, path, sizeof path);
     FILE *fout = fopen(path, "wt");
+    imsame_sweep_job swj;
+    FILE *fsweep[IMSAME_SWEEP_ENTRIES] = {NULL};
+    uint64_t sweep_accepted[IMSAME_SWEEP_ENTRIES] = {0};
+    int sweep_rc[IMSAME_SWEEP_ENTRIES] = {0};
+    if (G.sw.n) {
+        open_entries(u, fsweep);
+        swj.n = G.sw.n;
+        swj.coverage = G.sw.coverage;
+        swj.identity = G.sw.identity;
+        swj.out = fsweep;
+        swj.accepted = sweep_accepted;
+        swj.rc = sweep_rc;
+        jo.sweep = &swj;
+    }
     const double t0 = now_s();
     uint64_t accepted = 0;
     char err[300];
@@ -323,9 +380,20 @@ static int run_unit(worker *w, unit *u) {
         }
         if (fout) fclose(fout);
         fout = fopen(path, "wt");
+        if (G.sw.n) open_entries(u, fsweep);
         rc = imsame_run_job(q, db, &jo, fout, &w->ctx, &accepted, err, sizeof err);
     }
     if (fout) fclose(fout);
+    /* entry files are kept only for entries whose records are complete: none of a failed unit, none of an entry that
+       stopped on the read size */
+    for (int i = 0; i < G.sw.n; i++) {
+        if (fsweep[i]) fclose(fsweep[i]);
+        if (rc || sweep_rc[i]) {
+            char p[4096];
+            entry_path(u, i + 1, p, sizeof p);
+            unlink(p);
+        }
+    }
     if (rc == IMSAME_EREADSIZE) return unit_fail(u, "Read size reached for gapped alignment.");
     if (rc) {
         snprintf(msg, sizeof msg, "GPU hot path failed: %s%s%s", imsame_gpu_strerror(rc), err[0] ? " / " : "", err);
@@ -335,12 +403,39 @@ static int run_unit(worker *w, unit *u) {
         w->tab[u->i] = 1;
         w->tables++;
     }
-    if (asprintf(&u->text,
-                 "[INFO] %s vs %s%s: %" PRIu64 " reads (%" PRIu64 ") from the query were found in the database (%" PRIu64
-                 "); Jaccard-index %Le; %.3f s\n",
-                 si->name, sj->name, u->rev ? " (reverse complement)" : "", accepted, q->n_seqs, db->n_seqs,
-                 (long double)accepted / ((db->n_seqs + q->n_seqs) - accepted), now_s() - t0) < 0)
+    const char *strand = u->rev ? " (reverse complement)" : "";
+    size_t text_len = 0;
+    FILE *t = open_memstream(&u->text, &text_len);
+    if (!t) return unit_fail(u, "Could not allocate memory for the report");
+    fprintf(t,
+            "[INFO] %s vs %s%s: %" PRIu64 " reads (%" PRIu64 ") from the query were found in the database (%" PRIu64
+            "); Jaccard-index %Le; %.3f s\n",
+            si->name, sj->name, strand, accepted, q->n_seqs, db->n_seqs,
+            (long double)accepted / ((db->n_seqs + q->n_seqs) - accepted), now_s() - t0);
+    int stops = 0;
+    for (int i = 0; i < G.sw.n; i++) {
+        if (sweep_rc[i]) { /* a separate run at this threshold would have stopped here */
+            fprintf(t, "ERR**** Read size reached for gapped alignment. ****\n");
+            stops++;
+            continue;
+        }
+        const uint64_t a = sweep_accepted[i];
+        fprintf(t,
+                "[INFO] %s vs %s%s sweep %d of %d (-coverage %s -identity %s): %" PRIu64 " reads (%" PRIu64
+                ") from the query were found in the database (%" PRIu64 "); Jaccard-index %Le\n",
+                si->name, sj->name, strand, i + 1, G.sw.n, G.sw.text[i][0], G.sw.text[i][1], a, q->n_seqs, db->n_seqs,
+                (long double)a / ((db->n_seqs + q->n_seqs) - a));
+    }
+    if (fclose(t)) {
+        free(u->text);
+        u->text = NULL;
         return unit_fail(u, "Could not allocate memory for the report");
+    }
+    if (stops) {
+        pthread_mutex_lock(&G.lock);
+        G.entry_stops += stops;
+        pthread_mutex_unlock(&G.lock);
+    }
     return 0;
 }
 
@@ -463,14 +558,20 @@ int main(int argc, char **av) {
     jo.gpus = 1;
     jo.trace = getenv("IMSAME_TRACE") != NULL;
     int n_gpus = 1, n_jobs = 0;
+    const char *sweep = NULL;
     for (int i = 7; i < argc; i++) {
         if (strcmp(av[i], "-device") == 0 && i + 1 < argc) jo.device = atoi(av[i + 1]);
         if (strcmp(av[i], "-gpus") == 0) n_gpus = count_arg(argc, av, i, "-gpus");
         if (strcmp(av[i], "-jobs") == 0) n_jobs = count_arg(argc, av, i, "-jobs");
+        if (strcmp(av[i], "-sweep") == 0 && i + 1 < argc) sweep = av[i + 1];
     }
     if (!n_jobs) n_jobs = n_gpus;
     if (jo.mincoverage <= 0) terror("Min-coverage must be larger than zero");
     if (jo.minidentity <= 0) terror("Min-identity must be larger than zero");
+    if (sweep) {
+        const char *e = imsame_parse_sweep(sweep, &G.sw);
+        if (e) terror(e);
+    }
 
     /* `ls -d DIR/<name>.EXT`: names ending in ".EXT", in collation order */
     DIR *d = opendir(dir);
@@ -517,9 +618,7 @@ int main(int argc, char **av) {
                 u->i = (int)i;
                 u->j = (int)j;
                 u->rev = rev;
-                char path[4096];
-                unit_path(u, path, sizeof path);
-                if (exists(path)) continue;
+                if (unit_done(u)) continue;
                 sm[i].uses[0]++;
                 sm[j].uses[0]++; /* (a reverse unit: the forward parse decides the device path, the forward set feeds it) */
                 if (rev) sm[j].uses[1]++;
@@ -564,12 +663,13 @@ int main(int argc, char **av) {
     }
     fprintf(stdout, "[INFO] %" PRIu64 " comparisons of %zu samples in %.3f s\n", G.done, n, now_s() - t_all);
     fflush(stdout);
+    const int exit_status = G.entry_stops ? 255 : 0; /* (-sweep) the status of the separate run that would have stopped */
     /* every output file is closed: as in IMSAME (imsame_main.c) the release of the device and host memory is left
        to the operating system unless IMSAME_FAST_EXIT=0 asks for the orderly one */
     const char *fast = getenv("IMSAME_FAST_EXIT");
     if (!(fast && fast[0] == '0')) {
         fflush(stderr);
-        _exit(0);
+        _exit(exit_status);
     }
     for (int w = 0; w < G.n_workers; w++) {
         for (int x = 0; x < (int)(2 * n); x++)
@@ -591,5 +691,5 @@ int main(int argc, char **av) {
     }
     free(sm);
     free(G.u);
-    return 0;
+    return exit_status;
 }

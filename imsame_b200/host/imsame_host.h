@@ -65,6 +65,15 @@ void imsame_build_imin(long double min_identity, uint16_t *imin);
  * when it passes those. */
 void imsame_build_sweep_tables(int n_sets, const long double *coverage, const long double *identity, uint16_t *lmin_sets,
                                uint16_t *imin_sets, uint16_t *lmin_all, uint16_t *imin_all);
+/* -sweep C1:I1[,C2:I2...] of the command lines (IMSAME, IMSAME_allvsall): up to IMSAME_SWEEP_ENTRIES pairs, each value
+ * a whole number as atof reads it and larger than zero.  Returns NULL, or the error text the command line reports. */
+#define IMSAME_SWEEP_ENTRIES (IMSAME_SWEEP_MAX - 1) /* set 0 is -coverage / -identity */
+typedef struct imsame_sweep_list {
+    int n;
+    long double coverage[IMSAME_SWEEP_ENTRIES], identity[IMSAME_SWEEP_ENTRIES];
+    char text[IMSAME_SWEEP_ENTRIES][2][64]; /* the values as given, for the summary lines */
+} imsame_sweep_list;
+const char *imsame_parse_sweep(const char *list, imsame_sweep_list *s);
 
 /* ---- output ---------------------------------------------------------------- */
 /* header line of a record, src/alignmentFunctions.c:167 */

@@ -179,12 +179,13 @@ static int write_sweep_records(imsame_ctx **ctx, const imsame_job_opts *o, const
     return rc;
 }
 
-/* o->sweep: the job's thresholds as set 0 of imsame_gpu_align_sweep, the sweep's entries as sets 1 .. n */
+/* o->sweep: the job's thresholds as set 0 of the sweep, the sweep's entries as sets 1 .. n; with o->q_sample / db_sample
+   imsame_gpu_align_samples_sweep, else imsame_gpu_align_sweep from the host buffers */
 static int sweep_job(const imsame_fasta *q, const imsame_fasta *db, const imsame_job_opts *o, const imsame_params *p,
                      int kmer, FILE *fout, imsame_ctx **ctx_cache, uint64_t *accepted_out, char *err, size_t errlen) {
     imsame_sweep_job *sw = o->sweep;
     const int n_sets = 1 + sw->n;
-    if (n_sets > IMSAME_SWEEP_MAX || o->gpus > 1 || o->rev || o->q_sample) return IMSAME_EARG;
+    if (n_sets > IMSAME_SWEEP_MAX || o->gpus > 1 || o->rev) return IMSAME_EARG;
     double tp = now_s();
     imsame_seqinfo qv, dv;
     imsame_fasta_view(q, &qv);
@@ -203,7 +204,10 @@ static int sweep_job(const imsame_fasta *q, const imsame_fasta *db, const imsame
     if (!ctx && (rc = imsame_gpu_create(&ctx, o->device))) { free(best); return rc; }
     if (ctx_cache) *ctx_cache = ctx;
     rc = imsame_gpu_set_kmer(ctx, kmer);
-    if (!rc) rc = imsame_gpu_align_sweep(ctx, &dv, &qv, ps, n_sets, best, set_rc, NULL);
+    if (!rc) {
+        if (o->q_sample && o->db_sample) rc = imsame_gpu_align_samples_sweep(ctx, o->db_sample, o->q_sample, ps, n_sets, best, set_rc, NULL);
+        else rc = imsame_gpu_align_sweep(ctx, &dv, &qv, ps, n_sets, best, set_rc, NULL);
+    }
     if (rc && err && errlen) snprintf(err, errlen, "%s", imsame_gpu_last_cuda_error(ctx));
     if (!rc) rc = set_rc[0];  /* the main set's read-size stop ends the job as without the sweep */
     if (!rc) {

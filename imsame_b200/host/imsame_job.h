@@ -22,8 +22,9 @@ typedef struct imsame_rev_job {
     int rc;            /* out: the reverse strand's result (the job returns the forward strand's) */
 } imsame_rev_job;
 
-/* More coverage/identity sets in the same run (IMSAME -sweep): sets 1 .. n of imsame_gpu_align_sweep, the job's own
- * thresholds being set 0, whose records and count the job reports as without a sweep.  One GPU, no samples, no rev. */
+/* More coverage/identity sets in the same run (IMSAME -sweep, IMSAME_allvsall -sweep): sets 1 .. n of
+ * imsame_gpu_align_samples_sweep (with the job's two samples) or imsame_gpu_align_sweep (host buffers), the job's own
+ * thresholds being set 0, whose records and count the job reports as without a sweep.  One GPU, no rev. */
 typedef struct imsame_sweep_job {
     int n;
     const long double *coverage, *identity; /* n each */
@@ -45,7 +46,7 @@ typedef struct imsame_job_opts {
     const imsame_sample *db_sample;
     /* optional (not with the samples): the reverse strand too, after the forward records are written */
     imsame_rev_job *rev;
-    /* optional (gpus == 1, not with the samples or rev): more threshold sets in the same run */
+    /* optional (gpus == 1, not with rev): more threshold sets in the same run */
     imsame_sweep_job *sweep;
 } imsame_job_opts;
 

@@ -48,18 +48,13 @@ static double now_s(void) {
     return (double)t.tv_sec + 1e-9 * (double)t.tv_nsec;
 }
 
-#define SWEEP_ENTRIES (IMSAME_SWEEP_MAX - 1) /* set 0 is -coverage / -identity */
-
 typedef struct {
     const char *query, *db, *out, *out_rev, *sweep;
     uint64_t n_threads;
     long double minevalue, mincoverage, minidentity;
     int igap, egap;
     int gpus, device, kmer;
-    /* -sweep, parsed */
-    int n_sweep;
-    long double sweep_cov[SWEEP_ENTRIES], sweep_id[SWEEP_ENTRIES];
-    char sweep_text[SWEEP_ENTRIES][2][64]; /* the values as given, for the summary lines */
+    imsame_sweep_list sw; /* -sweep, parsed */
 } cli_args;
 
 static void usage_and_exit(void) { /* src/IMSAME.c:526-538 */
@@ -78,43 +73,10 @@ static void usage_and_exit(void) { /* src/IMSAME.c:526-538 */
     exit(1);
 }
 
-/* one value of a -sweep entry: a whole number as atof reads it (strtod accepts exactly what atof converts) */
-static int sweep_value(const char *b, const char *e, char *text, long double *v) {
-    const size_t n = (size_t)(e - b);
-    if (n == 0 || n >= 64) return 0;
-    memcpy(text, b, n);
-    text[n] = 0;
-    char *end = NULL;
-    (void)strtod(text, &end);
-    if (end != text + n) return 0;
-    *v = (long double)atof(text); /* double first, then widened, like -coverage / -identity */
-    return 1;
-}
-
-static void parse_sweep(const char *list, cli_args *a) {
-    const char *at = list;
-    a->n_sweep = 0;
-    for (;;) {
-        const char *comma = strchr(at, ',');
-        const char *end = comma ? comma : at + strlen(at);
-        const char *colon = memchr(at, ':', (size_t)(end - at));
-        if (a->n_sweep == SWEEP_ENTRIES) terror("-sweep takes at most 15 coverage:identity pairs");
-        const int i = a->n_sweep;
-        if (!colon || !sweep_value(at, colon, a->sweep_text[i][0], &a->sweep_cov[i]) ||
-            !sweep_value(colon + 1, end, a->sweep_text[i][1], &a->sweep_id[i]))
-            terror("-sweep expects a list of coverage:identity pairs, e.g. -sweep 0.5:0.7,0.5:0.9");
-        if (a->sweep_cov[i] <= 0) terror("Min-coverage must be larger than zero");
-        if (a->sweep_id[i] <= 0) terror("Min-identity must be larger than zero");
-        a->n_sweep++;
-        if (!comma) break;
-        at = comma + 1;
-    }
-}
-
 static void parse_args(int argc, char **av, cli_args *a) {
     /* defaults: src/IMSAME.c:44-49 */
     a->query = a->db = a->out = a->out_rev = a->sweep = NULL;
-    a->n_sweep = 0;
+    a->sw.n = 0;
     a->n_threads = 4;
     a->minevalue = 1 / powl(10, 20);
     a->mincoverage = 0.5;
@@ -155,7 +117,8 @@ static void parse_args(int argc, char **av, cli_args *a) {
         }
     }
     if (a->sweep) {
-        parse_sweep(a->sweep, a);
+        const char *e = imsame_parse_sweep(a->sweep, &a->sw);
+        if (e) terror(e);
         if (a->gpus > 1) terror("-sweep runs on one GPU: it cannot be combined with -gpus above 1");
         if (a->out_rev) terror("-sweep cannot be combined with -out_rev");
     }
@@ -214,10 +177,10 @@ int main(int argc, char **av) {
         rl.path = a.db;
         rl.started = pthread_create(&rl.thread, NULL, rev_load_main, &rl) == 0;
     }
-    FILE *fout_sweep[SWEEP_ENTRIES];
+    FILE *fout_sweep[IMSAME_SWEEP_ENTRIES];
     memset(fout_sweep, 0, sizeof fout_sweep);
     if (fout != NULL)
-        for (int i = 0; i < a.n_sweep; i++) {
+        for (int i = 0; i < a.sw.n; i++) {
             char path[4096];
             snprintf(path, sizeof path, "%s.%d", a.out, i + 1);
             if ((fout_sweep[i] = fopen(path, "wt")) == NULL) terror("Could not open a -sweep output file");
@@ -279,13 +242,13 @@ int main(int argc, char **av) {
         jo.rev = &rj;
     }
     imsame_sweep_job sj;
-    uint64_t sweep_accepted[SWEEP_ENTRIES] = {0};
-    int sweep_rc[SWEEP_ENTRIES] = {0};
+    uint64_t sweep_accepted[IMSAME_SWEEP_ENTRIES] = {0};
+    int sweep_rc[IMSAME_SWEEP_ENTRIES] = {0};
     memset(&sj, 0, sizeof sj);
-    if (a.n_sweep) {
-        sj.n = a.n_sweep;
-        sj.coverage = a.sweep_cov;
-        sj.identity = a.sweep_id;
+    if (a.sw.n) {
+        sj.n = a.sw.n;
+        sj.coverage = a.sw.coverage;
+        sj.identity = a.sw.identity;
         sj.out = fout_sweep;
         sj.accepted = sweep_accepted;
         sj.rc = sweep_rc;
@@ -335,9 +298,9 @@ int main(int argc, char **av) {
                 (long double)rj.accepted / ((rdb->n_seqs + q.n_seqs) - rj.accepted));
     }
     int exit_status = 0;
-    for (int i = 0; i < a.n_sweep; i++) {
-        fprintf(stdout, "[INFO] Sweep %d of %d: -coverage %s -identity %s\n", i + 1, a.n_sweep, a.sweep_text[i][0],
-                a.sweep_text[i][1]);
+    for (int i = 0; i < a.sw.n; i++) {
+        fprintf(stdout, "[INFO] Sweep %d of %d: -coverage %s -identity %s\n", i + 1, a.sw.n, a.sw.text[i][0],
+                a.sw.text[i][1]);
         if (sweep_rc[i]) { /* that run's terror line (src/commonFunctions.c:10-13); the process ends with its status */
             printf("ERR**** Read size reached for gapped alignment. ****\n");
             exit_status = 255;
@@ -346,14 +309,14 @@ int main(int argc, char **av) {
         fprintf(stdout,
                 "[INFO] %" PRIu64 " reads (%" PRIu64 ") from the query were found in the database (%" PRIu64
                 ") at a minimum e-value of %Le and minimum coverage of %d%%.\n",
-                sweep_accepted[i], q.n_seqs, db.n_seqs, (long double)a.minevalue, (int)(100 * a.sweep_cov[i]));
+                sweep_accepted[i], q.n_seqs, db.n_seqs, (long double)a.minevalue, (int)(100 * a.sw.coverage[i]));
         fprintf(stdout, "[INFO] The Jaccard-index is: %Le\n",
                 (long double)sweep_accepted[i] / ((db.n_seqs + q.n_seqs) - sweep_accepted[i]));
     }
     fprintf(stdout, "[INFO] Deallocating heap memory.\n");
     if (fout != NULL) fclose(fout);
     if (fout_rev != NULL) fclose(fout_rev);
-    for (int i = 0; i < a.n_sweep; i++)
+    for (int i = 0; i < a.sw.n; i++)
         if (fout_sweep[i] != NULL) fclose(fout_sweep[i]);
     fflush(stdout);
     /* Everything the caller can observe is on disk / on stdout now: the process ends here and leaves the device

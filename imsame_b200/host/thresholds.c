@@ -13,6 +13,8 @@
  */
 #include "imsame_host.h"
 #include <math.h>
+#include <stdlib.h>
+#include <string.h>
 
 /* e = (long double)0.333 * t_len * db_total_len * expl(-0.275 * rawscore), rawscore = 4n as
  * uint64 -> long double; QF_KARLIN / QF_LAMBDA are double literals (src/alignmentFunctions.h:1-2) */
@@ -84,4 +86,38 @@ void imsame_build_sweep_tables(int n_sets, const long double *coverage, const lo
         for (uint64_t i = 0; i < nl; i++) if (l[i] > lmin_all[i]) lmin_all[i] = l[i];
         for (uint64_t i = 0; i < ni; i++) if (m[i] > imin_all[i]) imin_all[i] = m[i];
     }
+}
+
+/* one value of a -sweep entry: a whole number as atof reads it (strtod accepts exactly what atof converts) */
+static int sweep_value(const char *b, const char *e, char *text, long double *v) {
+    const size_t n = (size_t)(e - b);
+    if (n == 0 || n >= sizeof(((imsame_sweep_list *)0)->text[0][0])) return 0;
+    memcpy(text, b, n);
+    text[n] = 0;
+    char *end = NULL;
+    (void)strtod(text, &end);
+    if (end != text + n) return 0;
+    *v = (long double)atof(text); /* double first, then widened, like -coverage / -identity */
+    return 1;
+}
+
+const char *imsame_parse_sweep(const char *list, imsame_sweep_list *s) {
+    const char *at = list;
+    s->n = 0;
+    for (;;) {
+        const char *comma = strchr(at, ',');
+        const char *end = comma ? comma : at + strlen(at);
+        const char *colon = memchr(at, ':', (size_t)(end - at));
+        if (s->n == IMSAME_SWEEP_ENTRIES) return "-sweep takes at most 15 coverage:identity pairs";
+        const int i = s->n;
+        if (!colon || !sweep_value(at, colon, s->text[i][0], &s->coverage[i]) ||
+            !sweep_value(colon + 1, end, s->text[i][1], &s->identity[i]))
+            return "-sweep expects a list of coverage:identity pairs, e.g. -sweep 0.5:0.7,0.5:0.9";
+        if (s->coverage[i] <= 0) return "Min-coverage must be larger than zero";
+        if (s->identity[i] <= 0) return "Min-identity must be larger than zero";
+        s->n++;
+        if (!comma) break;
+        at = comma + 1;
+    }
+    return NULL;
 }

@@ -234,9 +234,9 @@ int imsame_gpu_align_revcomp(imsame_ctx *const *ctxs, int n, imsame_best *out, i
  *                        zeroed, the others are complete.  The call returns 0 when the run completed.
  *   stats:               one for the run (its n_accepted is set 0's), or NULL.
  * imsame_gpu_set_kmer / _set_passes / _set_nw_mode apply as to imsame_gpu_align; the context stays usable after
- * every error.  Device memory: 16 bytes per set and query read on top of imsame_gpu_align.  Not covered: databases
- * sharded over several GPUs, resident samples (imsame_gpu_align_samples), imsame_gpu_align_revcomp after a sweep
- * (IMSAME_ESTATE), and sweeping the e-value, the gaps or the seed length. */
+ * every error.  Device memory: 16 bytes per set and query read on top of imsame_gpu_align.  Resident samples:
+ * imsame_gpu_align_samples_sweep (below).  Not covered: databases sharded over several GPUs, imsame_gpu_align_revcomp
+ * after a sweep (IMSAME_ESTATE), and sweeping the e-value, the gaps or the seed length. */
 #define IMSAME_SWEEP_MAX 16
 int imsame_gpu_align_sweep(imsame_ctx *ctx, const imsame_seqinfo *db, const imsame_seqinfo *query,
                            const imsame_params *params, int n_sets, imsame_best *out, int *set_rc,
@@ -301,6 +301,14 @@ void imsame_gpu_sample_free(imsame_ctx *ctx, imsame_sample *s);
  * first use for (seed length, params->n_threads) and kept in the sample. */
 int imsame_gpu_align_samples(imsame_ctx *ctx, const imsame_sample *db, imsame_sample *query,
                              const imsame_params *params, imsame_best *out, imsame_stats *stats);
+/* imsame_gpu_align_sweep with both read sets resident: params, n_sets, out, set_rc and stats as there, block t equal,
+ * field by field, to imsame_gpu_align_samples with params[t]; argument checks as both (IMSAME_ELIMIT for a database of
+ * more than one segment).  Device memory: 16 bytes per set and query read on top of imsame_gpu_align_samples.  The
+ * query keeps its word table; afterwards imsame_gpu_align_revcomp returns IMSAME_ESTATE; after any error
+ * (IMSAME_ENOMEM included) the context and both samples stay usable. */
+int imsame_gpu_align_samples_sweep(imsame_ctx *ctx, const imsame_sample *db, imsame_sample *query,
+                                   const imsame_params *params, int n_sets, imsame_best *out, int *set_rc,
+                                   imsame_stats *stats);
 
 /* ---- winners-only traceback (src/alignmentFunctions.c:493-546) ---------- */
 /* For each accepted read of `best`, NW is recomputed on the device with one
