@@ -41,6 +41,29 @@ class Best(C.Structure):
 BEST_DTYPE = np.dtype([("db_seq", "<u8"), ("qpos_end", "<u8"), ("db_pos", "<u8"), ("length", "<u4"),
                        ("identities", "<u4"), ("accepted", "<u4"), ("reserved", "<u4")])
 
+# imsame_aln: the alignment of a record (imsame_gpu_align_traceback); [start, end) inside each read
+ALN_DTYPE = np.dtype([("score", "<i4"), ("q_start", "<u4"), ("q_end", "<u4"), ("db_start", "<u4"), ("db_end", "<u4"),
+                      ("matches", "<u4"), ("mismatches", "<u4"), ("gap_cols", "<u4")])
+CIGAR_OPS = "MIDNSHP=X"  # BAM operation codes: op word = length << 4 | code
+
+
+def cigar_string(ops, extended=True):
+    """CIGAR text of one record's op words; extended=False merges '=' and 'X' into 'M'"""
+    out, last, run = [], None, 0
+    for w in ops:
+        n, c = int(w) >> 4, CIGAR_OPS[int(w) & 15]
+        if not extended and c in "=X":
+            c = "M"
+        if c == last:
+            run += n
+            continue
+        if last is not None:
+            out.append(f"{run}{last}")
+        last, run = c, n
+    if last is not None:
+        out.append(f"{run}{last}")
+    return "".join(out)
+
 
 class Stats(C.Structure):
     _fields_ = [("n_query_kmers", C.c_uint64), ("n_db_kmers", C.c_uint64), ("n_hits", C.c_uint64),
@@ -68,7 +91,7 @@ SYMBOLS = ["imsame_gpu_create", "imsame_gpu_destroy", "imsame_gpu_strerror", "im
            "imsame_gpu_db_revcomp", "imsame_gpu_align_revcomp", "imsame_gpu_align_sweep",
            "imsame_gpu_sample_create", "imsame_gpu_sample_revcomp", "imsame_gpu_sample_free", "imsame_gpu_align_samples",
            "imsame_gpu_align_samples_sweep",
-           "imsame_gpu_traceback", "imsame_gpu_free", "imsame_gpu_host_alloc", "imsame_gpu_host_free"]
+           "imsame_gpu_traceback", "imsame_gpu_align_traceback", "imsame_gpu_free", "imsame_gpu_host_alloc", "imsame_gpu_host_free"]
 
 _lib = None
 
@@ -116,6 +139,8 @@ def lib():
                                           C.POINTER(C.c_float)]
         l.imsame_gpu_traceback.argtypes = [vp, C.POINTER(SeqInfo), C.POINTER(SeqInfo), C.POINTER(Params), vp, vp,
                                            C.POINTER(C.POINTER(C.c_uint32)), vp]
+        l.imsame_gpu_align_traceback.argtypes = [vp, C.POINTER(SeqInfo), C.POINTER(SeqInfo), C.POINTER(Params), C.c_int,
+                                                 vp, vp, vp, C.POINTER(C.POINTER(C.c_uint32))]
         l.imsame_gpu_set_nw_mode.argtypes = [vp, C.c_int]
         l.imsame_gpu_set_passes.argtypes = [vp, C.c_int]
         l.imsame_gpu_set_kmer.argtypes = [vp, C.c_int]
@@ -426,6 +451,30 @@ class Imsame:
         ops = np.ctypeslib.as_array(ops_p, shape=(max(n, 1),))[:n].copy()
         lib().imsame_gpu_free(C.cast(ops_p, C.c_void_p))
         return ops_off, ops, cell
+
+    def align_traceback(self, db, query, records, params=None, db_breaks=None):
+        """the alignment of every accepted record (imsame_gpu_align_traceback): `records` = what align() /
+        align_revcomp() / align_samples() returns (db: the database its db_seq indexes -- the reverse complement for
+        reverse-strand records), or the list of sets of a sweep.  Returns (aln ALN_DTYPE[n], cigar_off uint64[n+1],
+        cigar uint32[]) over the records (the sets one after the other); record k's CIGAR is
+        cigar_string(cigar[cigar_off[k]:cigar_off[k+1]])."""
+        params = params or make_params()
+        sets = list(records) if isinstance(records, (list, tuple)) else [records]
+        best = np.ascontiguousarray(np.concatenate([np.asarray(r, dtype=BEST_DTYPE) for r in sets]), dtype=BEST_DTYPE)
+        d, k1 = _seqinfo(db[0], db[1], db_breaks)
+        q, k2 = _seqinfo(query[0], query[1])
+        n = len(best)
+        if n != len(sets) * int(q.n_seqs):
+            raise ValueError(f"{n} records for {len(sets)} set(s) of {int(q.n_seqs)} query reads")
+        aln = np.zeros(n, dtype=ALN_DTYPE)
+        off = np.zeros(n + 1, dtype=np.uint64)
+        ops_p = C.POINTER(C.c_uint32)()
+        self._check(lib().imsame_gpu_align_traceback(self._h, C.byref(d), C.byref(q), C.byref(params), len(sets),
+                                                     best.ctypes.data, aln.ctypes.data, off.ctypes.data, C.byref(ops_p)))
+        total = int(off[n])
+        ops = np.ctypeslib.as_array(ops_p, shape=(max(total, 1),))[:total].copy()
+        lib().imsame_gpu_free(C.cast(ops_p, C.c_void_p))
+        return aln, off, ops
 
     # -- NW on explicit pairs
     def nw_batch(self, xs, ys, igap=5, egap=2):

@@ -14,6 +14,7 @@
 
 #include "../../include/imsame_gpu.h"
 #include "../host/imsame_host.h"
+#include "cigar.cuh"
 #include "nw.cuh"
 #include "nwp_launch.h"
 #include "qtable.cuh"
@@ -135,6 +136,7 @@ struct imsame_ctx {
     cudaEvent_t pin_ev[2] = {nullptr, nullptr};
     bool pin_busy[2] = {false, false};     // a copy out of the buffer has been enqueued (wait for pin_ev before refilling)
     int nw_grid[9] = {0};                 // by columns per lane (1..8)
+    int cigar_grid = 0;                   // cigar_kernel (imsame_gpu_align_traceback)
     int nwp_grid[NW_CLASSES + 1] = {0};   // by NW class
     bool in_align = false;  // imsame_gpu_align: upload phases belong to the same stats
     int nw_mode = 0;  // 0: packed-word kernel where pw_eligible() holds, 1: generic kernel only
@@ -1816,3 +1818,4 @@ int imsame_gpu_traceback(imsame_ctx *ctx, const imsame_seqinfo *db, const imsame
 #include "capi_sharded.inc"
 #include "capi_samples.inc"
 #include "capi_sweep.inc"
+#include "capi_cigar.inc"

@@ -133,10 +133,15 @@ IMS_HD NwLink nw_first_link(uint32_t xi, uint32_t y0) {
     return k;
 }
 
-// TB: additionally store one back-pointer code per cell for the winners-only traceback
+// TB = 1: additionally store one back-pointer code per cell for the winners-only traceback
 // (src/alignmentFunctions.c:459-471 xfrom/yfrom): 0 = diagonal, 0x8000|x = jump to the
 // column maximum (x, j-1), 0x4000|y = jump to the row maximum (i-1, y).
 constexpr uint16_t TB_DIAG = 0, TB_COL = 0x8000, TB_ROW = 0x4000, TB_MASK = 0x3FFF;
+// TB = 2 (cigar.cuh): four bits per cell instead, the S cells of the strip in one 32-bit word (cell c at bits 4c):
+// the choice (0 = diagonal, 1 = jump to the column maximum, 2 = jump to the row maximum) and whether the cell moved
+// the row maximum to column j-2 (:434-438) or the maximum of column j-1 to row i-2 (:476-480).  The jump targets are
+// where those bits were last set, so the walk finds them again without storing them.
+constexpr uint32_t TBN_DIAG = 0, TBN_COL = 1, TBN_ROW = 2, TBN_DIR = 3, TBN_UP = 4, TBN_UC = 8;
 
 // One row of the lane's strip.
 //   P1 = T[i-1] (read only), P2 = T[i-2] on entry, T[i] on exit (written in place)
@@ -145,17 +150,19 @@ constexpr uint16_t TB_DIAG = 0, TB_COL = 0x8000, TB_ROW = 0x4000, TB_MASK = 0x3F
 //   cl: slot of column Y1 inside a strip ((Y1 - 1 - jb) % S, the same for every lane);
 //   owns_last: this lane's strip holds column Y1.
 // Columns j > Y1 are padding: they only ever feed cells further right, never a real one.
-template <int S, bool TB = false>
+//   tbrow: TB = 1: the row's S codes (uint16_t); TB = 2: the row's 32-bit word of 4-bit codes (S <= 8)
+template <int S, int TB = 0>
 IMS_HD void nw_row(NwLane<S> &L, const NwRow<S> &P1, NwRow<S> &P2, const NwLink &in, NwLink &out, int i, int j0,
                    uint32_t mm, int igap, int egap, int X1, int Y1, int cl, bool owns_last, bool first_lane,
-                   uint16_t *tbrow = nullptr) {
+                   void *tbrow = nullptr) {
     const int lb = igap - egap;                        // L = mfs + (j - mfy) * egap + lb
     const int rb = ((i == 1) ? NW_NEG : igap) - egap;  // no R candidate on row 1 (:449)
     int mfs = in.mfs, mfy = in.mfy, mfp = in.mfp;
     int nt = in.a, np = in.ap;   // value that becomes slot c of the new row: T[i][j0-1+c]
     int t2 = in.b;               // T[i][j-2]
     int r2 = P1.g, rp2 = P1.gp;  // T[i-1][j-2]
-    uint32_t tbw[4] = {0u, 0u, 0u, 0u};  // TB, S = 8: the row's codes, two per word
+    uint32_t tbw[4] = {0u, 0u, 0u, 0u};  // TB = 1, S = 8: the row's codes, two per word
+    uint32_t nib = 0u;                   // TB = 2: the row's 4-bit codes
 #pragma unroll
     for (int c = 0; c < S; c++) {
         const int j = j0 + c;
@@ -184,16 +191,18 @@ IMS_HD void nw_row(NwLane<S> &L, const NwRow<S> &P1, NwRow<S> &P2, const NwLink 
         const bool is_d = (m == d);
         const bool is_r = r > l;
         const int pj = is_r ? pr : pl;
-        if (TB) {
+        if (TB == 1) {
             const uint32_t code = is_d ? TB_DIAG : (is_r ? (uint32_t)(TB_COL | L.mcx[c]) : (uint32_t)(TB_ROW | mfy));
             // S = 8 (the only strip width the traceback launches): the row's eight codes leave as ONE 16-byte store
             // (tbrow is 16-byte aligned: strips start at multiples of 8 columns, rows at multiples of 256); as eight
             // 2-byte stores from 32 lanes on 32 different rows every store instruction touched 32 sectors
             if (S == 8) { if (c & 1) tbw[c >> 1] |= code << 16; else tbw[c >> 1] = code; }
-            else tbrow[c] = (uint16_t)code;
+            else static_cast<uint16_t *>(tbrow)[c] = (uint16_t)code;
         }
         // column maximum of column j-1 absorbs T[i-2][j-1], strictly greater only (:476-480)
         const bool uc = o2 > L.mcs[c];
+        if (TB == 2)
+            nib |= ((is_d ? TBN_DIAG : (is_r ? TBN_COL : TBN_ROW)) | (up ? TBN_UP : 0u) | (uc ? TBN_UC : 0u)) << (4 * c);
         L.mcs[c] = uc ? o2 : L.mcs[c];
         L.mcx[c] = uc ? i - 2 : L.mcx[c];
         L.mcp[c] = uc ? o2p : L.mcp[c];
@@ -204,13 +213,14 @@ IMS_HD void nw_row(NwLane<S> &L, const NwRow<S> &P1, NwRow<S> &P2, const NwLink 
         nt = m + s;
         np = is_d ? pd : pj;
     }
-    if (TB && S == 8) {
+    if (TB == 1 && S == 8) {
 #if defined(__CUDA_ARCH__)
         *reinterpret_cast<uint4 *>(tbrow) = make_uint4(tbw[0], tbw[1], tbw[2], tbw[3]);
 #else
-        for (int c = 0; c < 8; c++) tbrow[c] = (uint16_t)(tbw[c >> 1] >> (16 * (c & 1)));
+        for (int c = 0; c < 8; c++) static_cast<uint16_t *>(tbrow)[c] = (uint16_t)(tbw[c >> 1] >> (16 * (c & 1)));
 #endif
     }
+    if (TB == 2) *static_cast<uint32_t *>(tbrow) = nib;
     P2.h[S] = nt;
     P2.p[S] = np;
     P2.g = in.b;

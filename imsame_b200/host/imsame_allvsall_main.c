@@ -11,7 +11,7 @@
  * processes for 8 samples and re-parses every file 14 times.
  *
  * usage: IMSAME_allvsall metagenomes_directory coverage similarity threads file_extension outpath
- *                        [-device D] [-gpus N] [-jobs J] [-sweep C1:I1[,C2:I2...]]
+ *                        [-device D] [-gpus N] [-jobs J] [-sweep C1:I1[,C2:I2...]] [-cigar]
  *   -device D   first CUDA device (default 0)
  *   -gpus N     use the devices D .. D+N-1 (default 1)
  *   -jobs J     comparisons in flight (default N): J worker threads, each with its own CUDA context, go
@@ -28,6 +28,9 @@
  *               for that unit and prints the reference's "ERR**** Read size reached for gapped alignment. ****" in
  *               place of the entry's line; the run goes on and ends with exit status 255.  A stop of the main
  *               thresholds fails the unit as without -sweep.
+ *   -cigar      every record's header line ends with " q_start q_end db_start db_end score CIGAR", as with IMSAME
+ *               -cigar (in X-Y.r.align, coordinates inside the reverse complement read); each worker traces its own
+ *               records on its own device.  Without it every file is unchanged.
  *
  * A unit is one output file (X, Y, strand); the canonical order is the script's loop order.  A free worker
  * takes the next pending unit, preferring one whose query sample's word table it holds, then one whose
@@ -564,6 +567,7 @@ int main(int argc, char **av) {
         if (strcmp(av[i], "-gpus") == 0) n_gpus = count_arg(argc, av, i, "-gpus");
         if (strcmp(av[i], "-jobs") == 0) n_jobs = count_arg(argc, av, i, "-jobs");
         if (strcmp(av[i], "-sweep") == 0 && i + 1 < argc) sweep = av[i + 1];
+        if (strcmp(av[i], "-cigar") == 0) jo.cigar = 1;
     }
     if (!n_jobs) n_jobs = n_gpus;
     if (jo.mincoverage <= 0) terror("Min-coverage must be larger than zero");

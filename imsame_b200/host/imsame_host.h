@@ -79,6 +79,9 @@ const char *imsame_parse_sweep(const char *list, imsame_sweep_list *s);
 /* header line of a record, src/alignmentFunctions.c:167 */
 int imsame_format_header(char *dst, uint64_t read, uint64_t db_seq, uint32_t length, uint32_t identities,
                          uint64_t ylen);
+/* -cigar: dst = the end of a header just written by imsame_format_header; its first line gains the columns
+ * " q_start q_end db_start db_end score CIGAR" of `a` (imsame_gpu_align_traceback).  Returns the bytes it grew by. */
+size_t imsame_format_cigar_columns(char *dst, const imsame_aln *a, const uint32_t *ops, uint64_t n_ops);
 /* alignment text from a device traceback (ops = run-length path from the best
  * cell back to the border, see csrc/traceback.cuh), src/alignmentFunctions.c:230-271,493-560.
  * Returns bytes written (without the terminating 0). dst needs 6*(xlen+ylen)+256 bytes. */

@@ -30,16 +30,21 @@ static void *ctx_main(void *arg) {
     return NULL;
 }
 
-/* one traceback on the GPU: the ops and cells of the accepted reads of a record array */
+/* one traceback on the GPU: the ops and cells of the accepted reads of a record array; with -cigar also their
+   alignments (imsame_gpu_align_traceback) */
 typedef struct {
-    uint64_t *ops_off;
-    uint32_t *ops, *cell;
+    uint64_t *ops_off, *cigar_off;
+    uint32_t *ops, *cell, *cigar;
+    imsame_aln *aln;
 } tb_layer;
 
 static void tb_layer_free(tb_layer *L) {
     imsame_gpu_free(L->ops);
+    imsame_gpu_free(L->cigar);
     free(L->ops_off);
     free(L->cell);
+    free(L->cigar_off);
+    free(L->aln);
     memset(L, 0, sizeof *L);
 }
 
@@ -54,6 +59,12 @@ static int tb_layer_run(imsame_ctx **ctx, const imsame_job_opts *o, const imsame
     L->ops_off = (uint64_t *)malloc((q->n_seqs + 1) * sizeof(uint64_t));
     L->cell = (uint32_t *)malloc(4 * q->n_seqs * sizeof(uint32_t));
     rc = (L->ops_off && L->cell) ? imsame_gpu_traceback(*ctx, &dv, &qv, p, best, L->ops_off, &L->ops, L->cell) : IMSAME_ENOMEM;
+    if (!rc && o->cigar) {
+        L->cigar_off = (uint64_t *)malloc((q->n_seqs + 1) * sizeof(uint64_t));
+        L->aln = (imsame_aln *)malloc(q->n_seqs * sizeof(imsame_aln));
+        rc = (L->cigar_off && L->aln) ? imsame_gpu_align_traceback(*ctx, &dv, &qv, p, 1, best, L->aln, L->cigar_off, &L->cigar)
+                                      : IMSAME_ENOMEM;
+    }
     if (rc) {
         if (err && errlen) snprintf(err, errlen, "%s", imsame_gpu_last_cuda_error(*ctx));
         tb_layer_free(L);
@@ -87,7 +98,8 @@ static int render_records(const imsame_job_opts *o, const imsame_fasta *qf, cons
 #pragma omp parallel for schedule(static, 1) num_threads(nt)
         for (int t = 0; t < nt; t++) {
             const uint64_t r0 = q.n_seqs * (uint64_t)t / (uint64_t)nt, r1 = q.n_seqs * (uint64_t)(t + 1) / (uint64_t)nt;
-            const size_t rec_max = 6 * (2 * (size_t)IMSAME_MAX_READ_SIZE) + 768;
+            /* -cigar: at most xlen + ylen ops of at most 5 characters and six numbers */
+            const size_t rec_max = (o->cigar ? 11 : 6) * (2 * (size_t)IMSAME_MAX_READ_SIZE) + 768;
             size_t cap = 1 << 20, len = 0;
             char *buf = (char *)malloc(cap);
             for (uint64_t r = r0; r < r1 && buf; r++) {
@@ -103,6 +115,8 @@ static int render_records(const imsame_job_opts *o, const imsame_fasta *qf, cons
                 const uint32_t xlen = (uint32_t)(db.start_pos[s + 1] - db.start_pos[s]);
                 const uint32_t ylen = (uint32_t)(q.start_pos[r + 1] - q.start_pos[r]);
                 len += (size_t)imsame_format_header(buf + len, r, s, best[r].length, best[r].identities, ylen);
+                if (o->cigar) len += imsame_format_cigar_columns(buf + len, &L->aln[r], L->cigar + L->cigar_off[r],
+                                                                 L->cigar_off[r + 1] - L->cigar_off[r]);
                 len += (size_t)imsame_render_alignment(buf + len, db.sequences + db.start_pos[s], xlen,
                                                        q.sequences + q.start_pos[r], ylen, L->cell[4 * r], L->cell[4 * r + 1],
                                                        L->ops + L->ops_off[r], L->ops_off[r + 1] - L->ops_off[r]);

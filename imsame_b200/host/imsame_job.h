@@ -48,6 +48,9 @@ typedef struct imsame_job_opts {
     imsame_rev_job *rev;
     /* optional (gpus == 1, not with rev): more threshold sets in the same run */
     imsame_sweep_job *sweep;
+    /* -cigar: every record's header line ends with the alignment of its pair (imsame_gpu_align_traceback):
+       " q_start q_end db_start db_end score CIGAR" (0-based, ends exclusive, '=' / 'X' / 'I' / 'D' ops) */
+    int cigar;
 } imsame_job_opts;
 
 /* Aligns every read of q against db and writes the records of the accepted reads to fout (may be

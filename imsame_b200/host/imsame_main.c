@@ -23,6 +23,11 @@
  *               (imsame_gpu_align_revcomp), otherwise the reverse parse is uploaded.  stdout gains two lines after
  *               the Jaccard index, the numbers the second process would print; -out is what the run without the
  *               flag writes.  (Not in --help, whose text is the reference's.)
+ *   -cigar      every record's header line ends with the alignment of its pair, computed on the GPU
+ *               (imsame_gpu_align_traceback): " q_start q_end db_start db_end score CIGAR", coordinates 0-based with
+ *               exclusive ends inside the query read and the database read (for -out_rev records: the reverse complement
+ *               read they name), CIGAR ops '=' 'X' 'I' (query bases against a gap) 'D' (database bases against a gap).
+ *               Also for the -sweep files.  Without the flag the output is unchanged.  (Not in --help either.)
  */
 #define _GNU_SOURCE
 #include <inttypes.h>
@@ -53,7 +58,7 @@ typedef struct {
     uint64_t n_threads;
     long double minevalue, mincoverage, minidentity;
     int igap, egap;
-    int gpus, device, kmer;
+    int gpus, device, kmer, cigar;
     imsame_sweep_list sw; /* -sweep, parsed */
 } cli_args;
 
@@ -86,6 +91,7 @@ static void parse_args(int argc, char **av, cli_args *a) {
     a->gpus = 1;
     a->device = 0;
     a->kmer = 12; /* FIXED_K, src/structs.h:15 */
+    a->cigar = 0;
     for (int i = 0; i < argc; i++) { /* the reference also scans av[0] and never skips values */
         const char *nxt = (i + 1 < argc) ? av[i + 1] : NULL;
         if (strcmp(av[i], "--help") == 0) usage_and_exit();
@@ -111,6 +117,7 @@ static void parse_args(int argc, char **av, cli_args *a) {
         if (strcmp(av[i], "-n_threads") == 0 && nxt) a->n_threads = (uint64_t)atoi(nxt);
         if (strcmp(av[i], "-gpus") == 0 && nxt) a->gpus = atoi(nxt);
         if (strcmp(av[i], "-device") == 0 && nxt) a->device = atoi(nxt);
+        if (strcmp(av[i], "-cigar") == 0) a->cigar = 1;
         if (strcmp(av[i], "-kmer") == 0 && nxt) {
             a->kmer = atoi(nxt);
             if (a->kmer < 4 || a->kmer > 16) terror("The seed length must be between 4 and 16");
@@ -232,6 +239,7 @@ int main(int argc, char **av) {
     jo.gpus = a.gpus;
     jo.kmer = a.kmer;
     jo.device = a.device;
+    jo.cigar = a.cigar;
     jo.trace = getenv("IMSAME_TRACE") != NULL; /* phase wall times on stderr (not part of the reference's output) */
     imsame_rev_job rj;
     memset(&rj, 0, sizeof rj);

@@ -29,6 +29,17 @@ int imsame_format_header(char *dst, uint64_t read, uint64_t db_seq, uint32_t len
                    (unsigned long long)ylen);
 }
 
+size_t imsame_format_cigar_columns(char *dst, const imsame_aln *a, const uint32_t *ops, uint64_t n_ops) {
+    /* dst holds the header of imsame_format_header, "...\n $$$$$$$ \n": the columns go before its first newline */
+    static const char tail[] = "\n $$$$$$$ \n";
+    const size_t lt = sizeof tail - 1;
+    char *w = dst - lt;
+    w += sprintf(w, " %u %u %u %u %d ", a->q_start, a->q_end, a->db_start, a->db_end, a->score);
+    for (uint64_t k = 0; k < n_ops; k++) w += sprintf(w, "%u%c", ops[k] >> 4, "MIDNSHP=X"[ops[k] & 15]);
+    memcpy(w, tail, lt + 1);
+    return (size_t)(w + lt - dst);
+}
+
 uint64_t imsame_render_alignment(char *dst, const unsigned char *X, uint32_t xlen, const unsigned char *Y,
                                  uint32_t ylen, uint32_t bx, uint32_t by, const uint32_t *ops, uint64_t n_ops) {
     /* path length and end cell */

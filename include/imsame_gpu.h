@@ -326,6 +326,40 @@ int imsame_gpu_traceback(imsame_ctx *ctx, const imsame_seqinfo *db, const imsame
                          uint32_t *cell_xy);
 void imsame_gpu_free(void *p);
 
+/* ---- the alignment of every accepted record: CIGAR + exact coordinates ------------------------------------
+ * A record says which pair passed; this says how the two reads align, so that a hit can be checked, fed to a
+ * variant caller or to any tool that reads CIGARs without aligning the pair again.  The pair's NW is recomputed on
+ * the device with the forward kernel's own cell function, with 4 bits per cell, and walked back from the best border
+ * cell (csrc/cigar.cuh: one warp per pair, batches sorted by matrix size, largest first).
+ *   db, query, params: as for the call that produced the records (params: igap, egap, db_seq_base); for records of
+ *                      imsame_gpu_align_revcomp / IMSAME -out_rev, db is the reverse complement database those
+ *                      records index (revComp's order), and every coordinate refers to its reads.
+ *   best:   n_sets x nq records (one array, or the n_sets blocks of a sweep); record k is query read k % nq.
+ *           A (read, db_seq) pair that several sets accepted is traced once.
+ *   aln:    n_sets x nq entries, zero for records that are not accepted.
+ *   cigar_off: n_sets x nq + 1 entries; the ops of record k are cigar[cigar_off[k] .. cigar_off[k + 1]), in alignment
+ *           order, as BAM encodes them: length << 4 | op, op 7 '=', 8 'X', 1 'I' (query bases against a gap),
+ *           2 'D' (database bases against a gap).  *cigar is malloc'ed by the library (free with imsame_gpu_free).
+ * The path and the score: the start column (on the first base of one of the reads) is aligned, every gap run is
+ * followed by an aligned column, and aln.score = 4 (=) - 4 (X) + sum over gap runs (igap + length * egap), the NW
+ * score of the record.  The record's length = columns - 1 (the start column is not counted), its identities = the
+ * '=' columns that are neither the start column nor the column right after a gap run.  Ties break as in the forward
+ * kernel (DESIGN.md §9.9): diagonal if D >= L and D >= R, else the column jump if R > L, else the row jump.
+ * Device memory per batch: a budget of 1 GiB of codes and op slices (IMSAME_TRACEBACK_BUDGET, bytes, overrides
+ * it); larger sets of hits run in several batches with the same results.
+ * IMSAME_EARG for a record whose db_seq is outside db or whose length / identities are not those of its pair (the
+ * wrong database, e.g. the forward one for reverse-strand records); IMSAME_EREADSIZE for a read of more than
+ * IMSAME_MAX_READ_SIZE bases.  The context stays usable after every error. */
+typedef struct imsame_aln {
+    int32_t score;
+    uint32_t q_start, q_end;   /* query read bases [q_start, q_end) */
+    uint32_t db_start, db_end; /* database read bases [db_start, db_end) */
+    uint32_t matches, mismatches, gap_cols;
+} imsame_aln;
+int imsame_gpu_align_traceback(imsame_ctx *ctx, const imsame_seqinfo *db, const imsame_seqinfo *query,
+                               const imsame_params *params, int n_sets, const imsame_best *best, imsame_aln *aln,
+                               uint64_t *cigar_off, uint32_t **cigar);
+
 /* pinned host memory helpers for callers that want full-speed copies */
 void *imsame_gpu_host_alloc(uint64_t bytes);
 void imsame_gpu_host_free(void *p);
