@@ -18,6 +18,7 @@ GPU_SO = os.environ.get("IMSAME_GPU_SO") or os.path.join(_HERE, "_lib", "libimsa
 
 KEY_NONE = 0x7FFFFFFFFFFFFFFF
 SWEEP_MAX = 16  # IMSAME_SWEEP_MAX
+KMERS_MAX = 13  # IMSAME_KMERS_MAX
 
 
 class SeqInfo(C.Structure):
@@ -90,7 +91,7 @@ SYMBOLS = ["imsame_gpu_create", "imsame_gpu_destroy", "imsame_gpu_strerror", "im
            "imsame_gpu_run_sharded", "imsame_gpu_align_shard", "imsame_gpu_align_sharded",
            "imsame_gpu_db_revcomp", "imsame_gpu_align_revcomp", "imsame_gpu_align_sweep",
            "imsame_gpu_sample_create", "imsame_gpu_sample_revcomp", "imsame_gpu_sample_free", "imsame_gpu_align_samples",
-           "imsame_gpu_align_samples_sweep",
+           "imsame_gpu_align_samples_sweep", "imsame_gpu_align_kmers",
            "imsame_gpu_traceback", "imsame_gpu_align_traceback", "imsame_gpu_free", "imsame_gpu_host_alloc", "imsame_gpu_host_free"]
 
 _lib = None
@@ -124,6 +125,8 @@ def lib():
                                        C.POINTER(Stats)]
         l.imsame_gpu_align_sweep.argtypes = [vp, C.POINTER(SeqInfo), C.POINTER(SeqInfo), vp, C.c_int, vp, vp,
                                              C.POINTER(Stats)]
+        l.imsame_gpu_align_kmers.argtypes = [vp, C.POINTER(SeqInfo), C.POINTER(SeqInfo), C.POINTER(Params), C.c_int, vp,
+                                             vp, vp, vp]
         l.imsame_gpu_set_query.argtypes = [vp, C.POINTER(SeqInfo), C.POINTER(Params)]
         l.imsame_gpu_set_db.argtypes = [vp, C.POINTER(SeqInfo)]
         l.imsame_gpu_run.argtypes = [vp, C.POINTER(Params), vp, vp, C.POINTER(Stats)]
@@ -307,6 +310,25 @@ class Imsame:
                                                  out.ctypes.data, codes.ctypes.data, C.byref(st)))
         self.nq = nq
         return [out[t * nq:(t + 1) * nq].copy() for t in range(n)], [int(c) for c in codes[:n]], st.as_dict()
+
+    def align_kmers(self, db, query, ks, params=None, db_breaks=None):
+        """one call, several seed lengths (imsame_gpu_align_kmers): ks = distinct seed lengths 4..16 (at most
+        KMERS_MAX).  Returns ([records per k], [IMSAME_OK or IMSAME_EREADSIZE per k], [stats dict per k]): entry t's
+        records are what set_kmer(ks[t]) + align() return; an entry whose code is not 0 has all-zero records and
+        stats.  The context's own seed length is unchanged afterwards."""
+        params = params or make_params()
+        d, k1 = _seqinfo(db[0], db[1], db_breaks)
+        q, k2 = _seqinfo(query[0], query[1])
+        n, nq = len(ks), int(q.n_seqs)
+        karr = np.ascontiguousarray(list(ks) or [0], dtype=np.int32)
+        out = np.zeros(max(n, 1) * nq, dtype=BEST_DTYPE)
+        codes = np.zeros(max(n, 1), dtype=np.int32)
+        sts = (Stats * max(n, 1))()
+        self._check(lib().imsame_gpu_align_kmers(self._h, C.byref(d), C.byref(q), C.byref(params), n, karr.ctypes.data,
+                                                 out.ctypes.data, codes.ctypes.data, C.cast(sts, C.c_void_p)))
+        self.nq = nq
+        return ([out[t * nq:(t + 1) * nq].copy() for t in range(n)], [int(c) for c in codes[:n]],
+                [sts[t].as_dict() for t in range(n)])
 
     # -- staged form
     def set_query(self, query, params=None):

@@ -15,6 +15,7 @@
 #include "../../include/imsame_gpu.h"
 #include "../host/imsame_host.h"
 #include "cigar.cuh"
+#include "kcache.cuh"
 #include "nw.cuh"
 #include "nwp_launch.h"
 #include "qtable.cuh"
@@ -890,6 +891,9 @@ int db_layout(imsame_ctx *ctx, const imsame_seqinfo *db) {
     (void)class_mask_of(db->start_pos, db->n_seqs, db->total_len, &mx);
     ctx->db_maxlen = mx;
     if (mx > EXT_MAX_READ) return IMSAME_ELIMIT;
+    uint64_t seg_max = SEG_MAX_BASES;
+    if (const char *e = getenv("IMSAME_TEST_SEG_BASES"))  // test hook: several segments from a small database
+        seg_max = std::min<uint64_t>(seg_max, std::max<uint64_t>(std::max<uint64_t>(mx, 1), strtoull(e, nullptr, 10)));
     std::vector<uint32_t> tmp;
     uint64_t r0 = 0, bi = 0;
     while (r0 < db->n_seqs) {
@@ -897,13 +901,13 @@ int db_layout(imsame_ctx *ctx, const imsame_seqinfo *db) {
         const uint64_t base = db->start_pos[r0];
         uint64_t r1;
         if (fixed) {
-            r1 = std::min<uint64_t>(db->n_seqs, r0 + SEG_MAX_BASES / fixed);
+            r1 = std::min<uint64_t>(db->n_seqs, r0 + seg_max / fixed);
         } else {
             uint64_t lo = r0 + 1, hi = db->n_seqs;  // largest r1 with start[r1] - base <= SEG_MAX
             while (lo < hi) {
                 const uint64_t mid = (lo + hi + 1) / 2;
                 const uint64_t e = mid < db->n_seqs ? db->start_pos[mid] : db->total_len;
-                if (e - base <= SEG_MAX_BASES) lo = mid; else hi = mid - 1;
+                if (e - base <= seg_max) lo = mid; else hi = mid - 1;
             }
             r1 = lo;
         }
@@ -1819,3 +1823,4 @@ int imsame_gpu_traceback(imsame_ctx *ctx, const imsame_seqinfo *db, const imsame
 #include "capi_samples.inc"
 #include "capi_sweep.inc"
 #include "capi_cigar.inc"
+#include "capi_kmers.inc"

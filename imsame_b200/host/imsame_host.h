@@ -74,6 +74,14 @@ typedef struct imsame_sweep_list {
     char text[IMSAME_SWEEP_ENTRIES][2][64]; /* the values as given, for the summary lines */
 } imsame_sweep_list;
 const char *imsame_parse_sweep(const char *list, imsame_sweep_list *s);
+/* -kmers K1[,K2...] of IMSAME: up to IMSAME_KMERS_ENTRIES distinct seed lengths 4..16, none equal to `kmer` (the run's
+ * own -kmer, entry 0 of imsame_gpu_align_kmers).  Returns NULL, or the error text the command line reports. */
+#define IMSAME_KMERS_ENTRIES (IMSAME_KMERS_MAX - 1)
+typedef struct imsame_kmer_list {
+    int n;
+    int k[IMSAME_KMERS_ENTRIES];
+} imsame_kmer_list;
+const char *imsame_parse_kmers(const char *list, int kmer, imsame_kmer_list *s);
 
 /* ---- output ---------------------------------------------------------------- */
 /* header line of a record, src/alignmentFunctions.c:167 */

@@ -242,6 +242,50 @@ static int sweep_job(const imsame_fasta *q, const imsame_fasta *db, const imsame
     return rc;
 }
 
+/* o->kmers: the job's seed length as entry 0, the list's as entries 1 .. n (imsame_gpu_align_kmers); the records of
+   every entry are traced together, a winner that several entries share once (write_sweep_records) */
+_Static_assert(IMSAME_KMERS_MAX <= IMSAME_SWEEP_MAX, "write_sweep_records takes every entry");
+static int kmers_job(const imsame_fasta *q, const imsame_fasta *db, const imsame_job_opts *o, const imsame_params *p,
+                     int kmer, FILE *fout, imsame_ctx **ctx_cache, uint64_t *accepted_out, char *err, size_t errlen) {
+    imsame_kmers_job *kj = o->kmers;
+    const int n_k = 1 + kj->n;
+    if (n_k > IMSAME_KMERS_MAX || o->gpus > 1 || o->rev || o->sweep || o->q_sample) return IMSAME_EARG;
+    double tp = now_s();
+    imsame_seqinfo qv, dv;
+    imsame_fasta_view(q, &qv);
+    imsame_fasta_view(db, &dv);
+    int ks[IMSAME_KMERS_MAX];
+    ks[0] = kmer;
+    for (int t = 1; t < n_k; t++) ks[t] = kj->k[t - 1];
+    const uint64_t nq = q->n_seqs;
+    imsame_best *best = (imsame_best *)calloc((size_t)n_k * nq, sizeof(imsame_best));
+    if (!best) return IMSAME_ENOMEM;
+    int k_rc[IMSAME_KMERS_MAX];
+    imsame_ctx *ctx = (ctx_cache && *ctx_cache) ? *ctx_cache : NULL;
+    int rc = IMSAME_OK;
+    if (!ctx && (rc = imsame_gpu_create(&ctx, o->device))) { free(best); return rc; }
+    if (ctx_cache) *ctx_cache = ctx;
+    rc = imsame_gpu_align_kmers(ctx, &dv, &qv, p, n_k, ks, best, k_rc, NULL);
+    if (rc && err && errlen) snprintf(err, errlen, "%s", imsame_gpu_last_cuda_error(ctx));
+    if (!rc) rc = k_rc[0]; /* the main entry's read-size stop ends the job as without the list */
+    if (!rc) {
+        if (o->trace) { fprintf(stderr, "[imsame] align (%d seed lengths) %.3f s\n", n_k, now_s() - tp); tp = now_s(); }
+        FILE *fouts[IMSAME_KMERS_MAX];
+        for (int t = 0; t < n_k; t++) {
+            uint64_t acc = 0;
+            for (uint64_t r = 0; r < nq; r++) acc += best[(uint64_t)t * nq + r].accepted;
+            if (t) { kj->accepted[t - 1] = acc; kj->rc[t - 1] = k_rc[t]; }
+            else *accepted_out = acc;
+            fouts[t] = t ? (kj->out ? kj->out[t - 1] : NULL) : fout;
+            if (k_rc[t] || acc == 0) fouts[t] = NULL;
+        }
+        rc = write_sweep_records(&ctx, o, q, db, p, best, n_k, fouts, err, errlen, &tp);
+    }
+    if (ctx && !(ctx_cache && *ctx_cache == ctx)) imsame_gpu_destroy(ctx);
+    free(best);
+    return rc;
+}
+
 /* the reverse strand (o->rev) on the contexts of the forward one: ctxs[0 .. ng) (ctxs == &ctx when ng == 1) */
 static int reverse_strand(imsame_ctx **ctxs, int ng, const imsame_job_opts *o, const imsame_fasta *q, imsame_params *p,
                           char *err, size_t errlen, double *tp) {
@@ -302,6 +346,10 @@ int imsame_run_job(const imsame_fasta *qf, const imsame_fasta *dbf, const imsame
     if (o->sweep) {
         free(best);
         return sweep_job(&q, &db, o, &p, kmer, fout, ctx_cache, accepted_out, err, errlen);
+    }
+    if (o->kmers) {
+        free(best);
+        return kmers_job(&q, &db, o, &p, kmer, fout, ctx_cache, accepted_out, err, errlen);
     }
 
     int ng = o->gpus < 1 ? 1 : o->gpus;

@@ -33,6 +33,17 @@ typedef struct imsame_sweep_job {
     int *rc;                                /* out: n, IMSAME_OK or IMSAME_EREADSIZE */
 } imsame_sweep_job;
 
+/* More seed lengths in the same run (IMSAME -kmers): entries 1 .. n of imsame_gpu_align_kmers from the host buffers, the
+ * job's own seed length being entry 0, whose records and count the job reports as without the list.  One GPU, no rev,
+ * no sweep, no samples. */
+typedef struct imsame_kmers_job {
+    int n;
+    const int *k;       /* n seed lengths */
+    FILE **out;         /* n files for the records (NULL, or NULL entries: count only) */
+    uint64_t *accepted; /* out: n */
+    int *rc;            /* out: n, IMSAME_OK or IMSAME_EREADSIZE */
+} imsame_kmers_job;
+
 typedef struct imsame_job_opts {
     uint64_t n_threads;
     long double minevalue, mincoverage, minidentity;
@@ -48,6 +59,8 @@ typedef struct imsame_job_opts {
     imsame_rev_job *rev;
     /* optional (gpus == 1, not with rev): more threshold sets in the same run */
     imsame_sweep_job *sweep;
+    /* optional (gpus == 1, host buffers, not with rev or sweep): more seed lengths in the same run */
+    imsame_kmers_job *kmers;
     /* -cigar: every record's header line ends with the alignment of its pair (imsame_gpu_align_traceback):
        " q_start q_end db_start db_end score CIGAR" (0-based, ends exclusive, '=' / 'X' / 'I' / 'D' ops) */
     int cigar;

@@ -27,7 +27,15 @@
  *               (imsame_gpu_align_traceback): " q_start q_end db_start db_end score CIGAR", coordinates 0-based with
  *               exclusive ends inside the query read and the database read (for -out_rev records: the reverse complement
  *               read they name), CIGAR ops '=' 'X' 'I' (query bases against a gap) 'D' (database bases against a gap).
- *               Also for the -sweep files.  Without the flag the output is unchanged.  (Not in --help either.)
+ *               Also for the -sweep and -kmers files.  Without the flag the output is unchanged.  (Not in --help either.)
+ *   -kmers K1[,K2...]
+ *               more seed lengths in the same run (imsame_gpu_align_kmers: the read sets are uploaded once and the NW
+ *               result of a pair that an earlier seed length aligned is reused): entry Ki's records go to <out>.k<Ki>,
+ *               what `IMSAME ... -kmer Ki -out F` writes to F.  -out and the existing stdout lines are what the run
+ *               without the flag writes; after the Jaccard index, each entry prints "[INFO] Seed length Ki" and its
+ *               two summary lines, or the read-size error line in their place (its file stays empty, exit status 255).
+ *               At most 12 distinct values 4..16 other than -kmer; one GPU, not with -sweep or -out_rev.
+ *               (Not in --help either.)
  */
 #define _GNU_SOURCE
 #include <inttypes.h>
@@ -54,12 +62,13 @@ static double now_s(void) {
 }
 
 typedef struct {
-    const char *query, *db, *out, *out_rev, *sweep;
+    const char *query, *db, *out, *out_rev, *sweep, *kmers;
     uint64_t n_threads;
     long double minevalue, mincoverage, minidentity;
     int igap, egap;
     int gpus, device, kmer, cigar;
     imsame_sweep_list sw; /* -sweep, parsed */
+    imsame_kmer_list kl;  /* -kmers, parsed */
 } cli_args;
 
 static void usage_and_exit(void) { /* src/IMSAME.c:526-538 */
@@ -80,8 +89,9 @@ static void usage_and_exit(void) { /* src/IMSAME.c:526-538 */
 
 static void parse_args(int argc, char **av, cli_args *a) {
     /* defaults: src/IMSAME.c:44-49 */
-    a->query = a->db = a->out = a->out_rev = a->sweep = NULL;
+    a->query = a->db = a->out = a->out_rev = a->sweep = a->kmers = NULL;
     a->sw.n = 0;
+    a->kl.n = 0;
     a->n_threads = 4;
     a->minevalue = 1 / powl(10, 20);
     a->mincoverage = 0.5;
@@ -100,6 +110,7 @@ static void parse_args(int argc, char **av, cli_args *a) {
         if (strcmp(av[i], "-out") == 0 && nxt) a->out = nxt;
         if (strcmp(av[i], "-out_rev") == 0 && nxt) a->out_rev = nxt;
         if (strcmp(av[i], "-sweep") == 0 && nxt) a->sweep = nxt;
+        if (strcmp(av[i], "-kmers") == 0 && nxt) a->kmers = nxt;
         if (strcmp(av[i], "-evalue") == 0 && nxt) {
             a->minevalue = (long double)atof(nxt); /* double first, then widened (:553) */
             if (a->minevalue < 0) terror("Min-e-value must be larger than zero");
@@ -128,6 +139,13 @@ static void parse_args(int argc, char **av, cli_args *a) {
         if (e) terror(e);
         if (a->gpus > 1) terror("-sweep runs on one GPU: it cannot be combined with -gpus above 1");
         if (a->out_rev) terror("-sweep cannot be combined with -out_rev");
+    }
+    if (a->kmers) {
+        const char *e = imsame_parse_kmers(a->kmers, a->kmer, &a->kl);
+        if (e) terror(e);
+        if (a->sweep) terror("-kmers cannot be combined with -sweep");
+        if (a->gpus > 1) terror("-kmers runs on one GPU: it cannot be combined with -gpus above 1");
+        if (a->out_rev) terror("-kmers cannot be combined with -out_rev");
     }
 }
 
@@ -191,6 +209,14 @@ int main(int argc, char **av) {
             char path[4096];
             snprintf(path, sizeof path, "%s.%d", a.out, i + 1);
             if ((fout_sweep[i] = fopen(path, "wt")) == NULL) terror("Could not open a -sweep output file");
+        }
+    FILE *fout_kmers[IMSAME_KMERS_ENTRIES];
+    memset(fout_kmers, 0, sizeof fout_kmers);
+    if (fout != NULL)
+        for (int i = 0; i < a.kl.n; i++) {
+            char path[4096];
+            snprintf(path, sizeof path, "%s.k%d", a.out, a.kl.k[i]);
+            if ((fout_kmers[i] = fopen(path, "wt")) == NULL) terror("Could not open a -kmers output file");
         }
 
     double t0 = now_s();
@@ -262,6 +288,18 @@ int main(int argc, char **av) {
         sj.rc = sweep_rc;
         jo.sweep = &sj;
     }
+    imsame_kmers_job kj;
+    uint64_t kmers_accepted[IMSAME_KMERS_ENTRIES] = {0};
+    int kmers_rc[IMSAME_KMERS_ENTRIES] = {0};
+    memset(&kj, 0, sizeof kj);
+    if (a.kl.n) {
+        kj.n = a.kl.n;
+        kj.k = a.kl.k;
+        kj.out = fout_kmers;
+        kj.accepted = kmers_accepted;
+        kj.rc = kmers_rc;
+        jo.kmers = &kj;
+    }
     char err[300];
     imsame_ctx *ctx = NULL;
     if (booting) {
@@ -321,11 +359,27 @@ int main(int argc, char **av) {
         fprintf(stdout, "[INFO] The Jaccard-index is: %Le\n",
                 (long double)sweep_accepted[i] / ((db.n_seqs + q.n_seqs) - sweep_accepted[i]));
     }
+    for (int i = 0; i < a.kl.n; i++) {
+        fprintf(stdout, "[INFO] Seed length %d\n", a.kl.k[i]);
+        if (kmers_rc[i]) { /* (as for -sweep) */
+            printf("ERR**** Read size reached for gapped alignment. ****\n");
+            exit_status = 255;
+            continue;
+        }
+        fprintf(stdout,
+                "[INFO] %" PRIu64 " reads (%" PRIu64 ") from the query were found in the database (%" PRIu64
+                ") at a minimum e-value of %Le and minimum coverage of %d%%.\n",
+                kmers_accepted[i], q.n_seqs, db.n_seqs, (long double)a.minevalue, (int)(100 * a.mincoverage));
+        fprintf(stdout, "[INFO] The Jaccard-index is: %Le\n",
+                (long double)kmers_accepted[i] / ((db.n_seqs + q.n_seqs) - kmers_accepted[i]));
+    }
     fprintf(stdout, "[INFO] Deallocating heap memory.\n");
     if (fout != NULL) fclose(fout);
     if (fout_rev != NULL) fclose(fout_rev);
     for (int i = 0; i < a.sw.n; i++)
         if (fout_sweep[i] != NULL) fclose(fout_sweep[i]);
+    for (int i = 0; i < a.kl.n; i++)
+        if (fout_kmers[i] != NULL) fclose(fout_kmers[i]);
     fflush(stdout);
     /* Everything the caller can observe is on disk / on stdout now: the process ends here and leaves the device
        memory, the pinned buffers and the parsed reads to the operating system instead of releasing them piece by

@@ -121,3 +121,25 @@ const char *imsame_parse_sweep(const char *list, imsame_sweep_list *s) {
     }
     return NULL;
 }
+
+const char *imsame_parse_kmers(const char *list, int kmer, imsame_kmer_list *s) {
+    const char *at = list;
+    s->n = 0;
+    for (;;) {
+        const char *comma = strchr(at, ',');
+        const char *end = comma ? comma : at + strlen(at);
+        if (s->n == IMSAME_KMERS_ENTRIES) return "-kmers takes at most 12 seed lengths";
+        long v = 0;
+        const char *c = at;
+        for (; c < end && *c >= '0' && *c <= '9' && c - at < 3; c++) v = 10 * v + (*c - '0');
+        if (c == at || c != end) return "-kmers expects a list of seed lengths, e.g. -kmers 8,10,14";
+        if (v < 4 || v > 16) return "The seed length must be between 4 and 16";
+        if (v == kmer) return "-kmers must not repeat a seed length or give the -kmer one";
+        for (int i = 0; i < s->n; i++)
+            if (s->k[i] == v) return "-kmers must not repeat a seed length or give the -kmer one";
+        s->k[s->n++] = (int)v;
+        if (!comma) break;
+        at = comma + 1;
+    }
+    return NULL;
+}

@@ -236,11 +236,43 @@ int imsame_gpu_align_revcomp(imsame_ctx *const *ctxs, int n, imsame_best *out, i
  * imsame_gpu_set_kmer / _set_passes / _set_nw_mode apply as to imsame_gpu_align; the context stays usable after
  * every error.  Device memory: 16 bytes per set and query read on top of imsame_gpu_align.  Resident samples:
  * imsame_gpu_align_samples_sweep (below).  Not covered: databases sharded over several GPUs, imsame_gpu_align_revcomp
- * after a sweep (IMSAME_ESTATE), and sweeping the e-value, the gaps or the seed length. */
+ * after a sweep (IMSAME_ESTATE), and sweeping the e-value or the gaps (several seed lengths:
+ * imsame_gpu_align_kmers, below). */
 #define IMSAME_SWEEP_MAX 16
 int imsame_gpu_align_sweep(imsame_ctx *ctx, const imsame_seqinfo *db, const imsame_seqinfo *query,
                            const imsame_params *params, int n_sets, imsame_best *out, int *set_rc,
                            imsame_stats *stats);
+
+/* ---- several seed lengths in one call ---------------------------------------------------------------
+ * The low-identity sweeps that compare metagenomes at several seed lengths run one IMSAME process per k.  The NW of a
+ * candidate pair aligns the two whole reads (src/alignmentFunctions.c:389-489), wherever the seed was: its result does
+ * not depend on k, and seeds of different lengths keep finding the same (query read, database read) pairs.  This call
+ * uploads and packs both read sets once and runs one entry per seed length, in the order given; each entry builds
+ * the word table of its k (the previous entry's is freed first) and takes the NW result of every pair an earlier
+ * entry aligned from a device cache that lives for the call only (csrc/kcache.cuh).
+ *   ks[0 .. n_k):  distinct seed lengths, 4 <= k <= 16; 1 <= n_k <= IMSAME_KMERS_MAX.
+ *   out:           n_k x nq records; block t (out + t * nq) equals, field by field, what imsame_gpu_set_kmer(ks[t]) +
+ *                  imsame_gpu_align(db, query, params) return on the same context, scan plan included (one pass or
+ *                  early words first, imsame_gpu_set_passes).
+ *   k_rc[t]:       IMSAME_OK, or IMSAME_EREADSIZE exactly where that separate run stops with "Read size reached for
+ *                  gapped alignment."; that entry's block (and stats) is zeroed, the others are complete.  The call
+ *                  returns 0 when every entry ran.
+ *   stats:         n_k entries or NULL.  n_query_kmers, n_db_kmers, n_hits, n_evalue_pass, n_pairs and n_accepted equal
+ *                  the separate run's; n_pairs_dp and n_cells count the pairs whose NW this entry computed (a pair
+ *                  taken from the cache is not counted).  Phase times and launches are the entry's own (entry 0's
+ *                  include the uploads).
+ * IMSAME_EARG for n_k out of range, a k out of range, a repeated k, or NULL ks / out / k_rc.  The context keeps its
+ * own seed length (imsame_gpu_set_kmer); imsame_gpu_set_passes / _set_nw_mode apply to every entry; afterwards
+ * imsame_gpu_align_revcomp returns IMSAME_ESTATE; after every error (IMSAME_ENOMEM included) the context takes the
+ * next call.  Device memory: the largest k's word table (imsame_gpu_set_kmer), 16 bytes per candidate pair of an
+ * entry, and the cache: 12 bytes per slot, at most half of them used, one slot per pair aligned so far.
+ * Not covered: databases sharded over several GPUs, resident samples, and combining it with a coverage / identity
+ * sweep (imsame_gpu_align_sweep). */
+#define IMSAME_KMERS_MAX 13 /* every seed length 4..16 once */
+int imsame_gpu_align_kmers(imsame_ctx *ctx, const imsame_seqinfo *db, const imsame_seqinfo *query,
+                           const imsame_params *params, int n_k, const int *ks,
+                           imsame_best *out /* n_k x nq */, int *k_rc /* n_k */,
+                           imsame_stats *stats /* n_k entries or NULL */);
 
 /* ---- NW on explicit pairs (src/alignmentFunctions.c:389-560 in isolation) */
 /* X[i] / Y[i]: ASCII reads; out5[i*5..] = score, bx, by, length, identities */
